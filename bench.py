@@ -10,7 +10,7 @@ north_star's target sentence names: "synthetic R1CS circuit 2^20 multipliers (MS
 The circuit is the reference's test_merkle_tree_gadget_512: MerkleTree256 over 512 committed leaves (511 two-block MiMC nodes).
 A proof = 512 Pedersen commits, 3 commitment MSMs of 2n+1 / n+1 / 2n+1 points, polynomial phase, 20 IPP rounds.
 A step = P proofs, one per concurrent prover of the GPU (own host thread + bpg_ctx + witness each; P is in `config`);
-the P * steps proofs of the timed region are handed out to free-running provers, so the sequential host-side Merlin
+every prover runs through its `steps` proofs of the timed region without waiting for the others, so the sequential host-side Merlin
 TranscriptRng of one proof (2n draws, ~0.7 s of one core at this size; the streams of concurrent provers share SIMD
 lanes) overlaps the device work of the others.  Every rank runs its own provers (weak scaling, no data-path collective).
 
@@ -23,6 +23,11 @@ lanes) overlaps the device work of the others.  Every rank runs its own provers 
 Extras: MSM sweeps 2^16..2^22 with the oracle's Mpoints/s beside every point, MiMC, BASELINE configs[1] and [4]
 (batch verification of 8192 set_membership / less_than proofs, sharded by rank, verdicts == oracle), and for N > 1 the
 oracle-parity checks of the sharded MSM and the sharded prover.
+
+--dump-outputs DIR: after the run, DIR/proofs.npy and DIR/commitments.npy hold what the timed region (`value`; for
+`--impl reference` its oracle proofs) returned in its last step: one row per prover of rank 0, the proof bytes and the
+commitment bytes V as float32 values 0..255.  The inputs of that step depend on the arguments only, so two builds of the
+project can be compared output for output.
 
 The reference itself (Rust) cannot be built in this image; `--impl reference` times the oracle port.
 """
@@ -123,6 +128,18 @@ def oracle_prove(inst, cap, ext, threads):
     return time.perf_counter() - t0, proof, V
 
 
+def dump_outputs(path, outputs):
+    """--dump-outputs: `outputs` = the (proof, V) byte strings of one step, one per prover, written as float32 arrays of byte
+    values (exact); the rows beyond the first that fit in 64 MB are left out"""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    row_bytes = 4 * (len(outputs[0][0]) + len(outputs[0][1]))
+    outputs = outputs[:max(1, (64 << 20) // row_bytes)]
+    for name, col in (("proofs", 0), ("commitments", 1)):
+        rows = np.array([np.frombuffer(o[col], dtype=np.uint8) for o in outputs], dtype=np.float32)
+        np.save(os.path.join(path, name + ".npy"), rows)
+
+
 def run_reference(args):
     """Reference arm: the reference's CPU algorithm for the same path on the host cores (oracle port, OpenMP on all cores; the
     Rust crate cannot be built here).  A complete 2^20 proof takes the oracle ~20 s on 16 cores, so every step is a bounded
@@ -147,8 +164,10 @@ def run_reference(args):
         oracle_prove(inst, cap, bytes(32), cores)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        oracle_prove(inst, cap, bytes(32), cores)
+        _, proof, V = oracle_prove(inst, cap, bytes(32), cores)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [(proof, V)])
     v = args.steps / dt / scale
     sample = ("every step = 1 complete oracle proof of a %d-multiplier circuit of the same family (N = %d), OpenMP on all host cores; "
               "value = sample proofs/s / %.2f (cost linear in the multiplier count)" % (inst["n"], cap, scale)) if not full else \
@@ -559,7 +578,7 @@ class ProverLane:
 
 
 class LaneSet:
-    """P free-running provers on one GPU; timed(flags, resident, steps) runs P * steps proofs handed out one at a time"""
+    """P free-running provers on one GPU; timed(flags, resident, steps) runs P * steps proofs, one per prover and step"""
 
     def __init__(self, bpg, gadgets, device, insts, cap, rank):
         from concurrent.futures import ThreadPoolExecutor
@@ -567,49 +586,40 @@ class LaneSet:
         self.P = len(self.lanes)
         self.pool = ThreadPoolExecutor(max_workers=self.P)
         self.rank = rank
-        self.tickets = {"next": 0, "total": 0, "lock": threading.Lock()}
         self.host_cpu_ms = 0.0
         self.region = 0
         self.prefetch = True
+        self.last = [None] * self.P  # (proof, V) of every lane's proof in the last step of the latest region
 
     def _ext(self, ticket):
         # every proof of the run gets its own 32 bytes standing for the reference's thread_rng draw
         return hashlib.sha256(b"bench ext %d %d %d" % (self.rank, self.region, ticket)).digest()
 
-    def _take(self):
-        with self.tickets["lock"]:
-            if self.tickets["next"] >= self.tickets["total"]:
-                return None
-            tk = self.tickets["next"]
-            self.tickets["next"] += 1
-            return tk
-
-    def _lane_run(self, ln, flags, resident):
-        """A lane works through tickets.  It always holds its NEXT ticket as well and hands that proof's opening to the library
-        (bpg_r1cs_prove_prefetch) before proving the current one, so the sequential transcript-RNG stream of proof k+1 is drawn
-        by a background host thread while proof k is on the device."""
-        time.sleep(0.001 * self.lanes.index(ln))  # staggered start (inside the timed region)
-        cur = self._take()
-        while cur is not None:
-            nxt = self._take()
-            if nxt is not None and self.prefetch:
-                ln.circ.prefetch(ln.inst, self._ext(nxt), flags)
-            ln.prove(self._ext(cur), flags, resident)
-            cur = nxt
+    def _lane_run(self, k, flags, resident, steps):
+        """Lane k proves tickets k, k + P, ... (ticket s * P + k in step s), so every proof's witness and ext_rng32 are the same
+        from run to run.  Before proving a ticket it hands the opening of its NEXT one to the library (bpg_r1cs_prove_prefetch),
+        so the sequential transcript-RNG stream of that proof is drawn by a background host thread while this one is on the device."""
+        ln = self.lanes[k]
+        time.sleep(0.001 * k)  # staggered start (inside the timed region)
+        tickets = range(k, self.P * steps, self.P)
+        for i, cur in enumerate(tickets):
+            if i + 1 < len(tickets) and self.prefetch:
+                ln.circ.prefetch(ln.inst, self._ext(tickets[i + 1]), flags)
+            self.last[k] = ln.prove(self._ext(cur), flags, resident)
 
     def timed(self, flags, resident, steps):
         """-> (ms, launches).  The region is bracketed by a sync of every context on both sides; device time by CUDA events on
         lane 0's stream, wall clock beside it, the larger of the two is reported."""
         self.region += 1
+        self.last = [None] * self.P
         for ln in self.lanes:
             ln.ctx.sync()
         l0 = sum(ln.ctx.launch_count() for ln in self.lanes)
-        self.tickets["next"], self.tickets["total"] = 0, self.P * steps
         ctx = self.lanes[0].ctx
         ctx.event_record(2)
         c0 = os.times()
         t0 = time.perf_counter()
-        list(self.pool.map(lambda ln: self._lane_run(ln, flags, resident), self.lanes))
+        list(self.pool.map(lambda k: self._lane_run(k, flags, resident, steps), range(self.P)))
         for ln in self.lanes:
             ln.ctx.sync()
         ctx.event_record(3)
@@ -674,6 +684,7 @@ def run_ours(args):
     ctx.prof_enable(True)
     barrier_max(dist, local, 0.0)
     ms_value, launches = lanes.timed(RES, True, args.steps)
+    last_step = lanes.last
     ms_value = barrier_max(dist, local, ms_value)
     cpu_ms_value = lanes.host_cpu_ms
     nl_c, kms_c, pairs_c = ctx.prof_read()   # lane 0's launches inside the timed region: they share the GPU with the other lanes
@@ -847,6 +858,8 @@ def run_ours(args):
                                                          "interval includes the time its blocks wait for slots behind every other prover's kernels" % (P - 1)}},
                 "cpu_baseline": cpu, "clocks": sampler.summary()}
         line.update(extras)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_step)
         _emit(json.dumps(line))
     ctx0.close()
     if dist is not None:
@@ -892,6 +905,7 @@ def main():
     ap.add_argument("--quick", action="store_true", help="small MSM sweep only, no config extras")
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the timed region's last-step outputs to DIR/*.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -29,6 +29,29 @@ def test_reference_arm_prints_one_contract_line():
     assert d["e2e"] == {"value": d["value"], "unit": "proofs/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+def test_reference_arm_dumps_last_step_outputs(tmp_path):
+    """--dump-outputs writes the proof and commitments the timed steps computed, as float32 byte values that equal a fresh oracle
+    proof of the same instance"""
+    import numpy as np
+    env = dict(os.environ, RANK="0", WORLD_SIZE="1")
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
+                          "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600, env=env, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    sys.path.insert(0, ROOT)
+    import bench
+    import oracle_lib as ol
+    from bulletproofs_gadgets_b200 import gadgets
+    inst = gadgets.merkle_tree_instances(bench.REF_SAMPLE_LEAVES, [None], trace_on_device=False)[0]
+    try:
+        _, proof, V = bench.oracle_prove(inst, 1 << 16, bytes(32), os.cpu_count() or 1)
+    finally:
+        ol.lib().bpo_set_threads(1)
+    for name, want in (("proofs", proof), ("commitments", V)):
+        got = np.load(str(tmp_path / (name + ".npy")))
+        assert got.dtype == np.float32 and got.shape == (1, len(want))
+        assert bytes(got[0].astype(np.uint8)) == want
+
+
 def test_reference_arm_is_silent_on_other_ranks():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "0"],
