@@ -52,6 +52,9 @@ SYMBOLS = {
     "bpg_witness_eval": (_i32, [_vp, _sz, _sz, _u32p, _u32p, _u8p, _u8p, _u8p, _u8p, _u8p]),
     "bpg_r1cs_prove": (C.c_long, [_vp, _vp, _u8p, _sz, _u8p, _u8p, _u8p, _u8p, _u8p, _u8p, C.c_uint, _u8p, _u8p, _sz]),
     "bpg_r1cs_prove_prefetch": (_i32, [_vp, _vp, _u8p, _sz, _u8p, _u8p, _u8p, C.c_uint]),
+    "bpg_r1cs_prove_batch": (_i32, [_vp, _sz, C.POINTER(_vp), C.POINTER(C.c_char_p), C.POINTER(_sz), C.POINTER(C.c_char_p), C.POINTER(C.c_char_p),
+                                    C.POINTER(C.c_char_p), C.POINTER(C.c_char_p), C.POINTER(C.c_char_p), _u8p, C.c_uint, C.POINTER(_vp), C.POINTER(_vp),
+                                    C.POINTER(_sz), C.POINTER(_sz)]),
     "bpg_r1cs_verify": (_i32, [_vp, _vp, _u8p, _sz, _u8p, _u8p, _sz, _u8p, C.c_uint, C.POINTER(_i32)]),
     "bpg_r1cs_verify_batch": (_i32, [_vp, _sz, C.POINTER(_vp), C.POINTER(C.c_char_p), C.POINTER(_sz), C.POINTER(C.c_char_p), C.POINTER(C.c_char_p),
                                      C.POINTER(_sz), _u8p, C.c_uint, C.POINTER(_i32)]),

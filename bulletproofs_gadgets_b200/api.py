@@ -158,6 +158,26 @@ class Context:
         raw = out.raw  # (.raw copies the whole buffer: take it once)
         return [raw[32 * i:32 * i + 32] for i in range(n)], (tr.raw if trace else None)
 
+    # ---- batched proving
+    def prove_batch(self, items, flags=0):
+        """items: list of (circuit handle (c_void_p), label bytes, aL, aR, aO, v, v_blinding (n or m x 32 bytes each), ext_rng32)
+        -> list of (proof bytes, V bytes), entry i being exactly what bpg_r1cs_prove returns for item i"""
+        n = len(items)
+        if n == 0:
+            return []
+        ms = [len(it[5] or b"") // 32 for it in items]
+        cap = 1 + 32 * (14 + 64 + 2)
+        ptr = lambda xs: (C.c_char_p * n)(*xs)
+        proofs = [C.create_string_buffer(cap) for _ in range(n)]
+        Vs = [C.create_string_buffer(32 * max(1, m)) for m in ms]
+        lens = (C.c_size_t * n)()
+        self.check(self.lib.bpg_r1cs_prove_batch(
+            self.h, n, (C.c_void_p * n)(*[it[0] for it in items]), ptr([it[1] for it in items]), (C.c_size_t * n)(*[len(it[1]) for it in items]),
+            ptr([it[2] for it in items]), ptr([it[3] for it in items]), ptr([it[4] for it in items]), ptr([it[5] for it in items]),
+            ptr([it[6] for it in items]), b"".join(it[7] for it in items), flags, (C.c_void_p * n)(*[C.addressof(b) for b in Vs]),
+            (C.c_void_p * n)(*[C.addressof(b) for b in proofs]), (C.c_size_t * n)(*([cap] * n)), lens))
+        return [(proofs[i].raw[:lens[i]], Vs[i].raw[:32 * ms[i]]) for i in range(n)]
+
     # ---- batch verification
     def verify_batch(self, items, flags=0):
         """items: list of (circuit handle (c_void_p), label bytes, V bytes, proof bytes, ext_rng32) -> list of bool,
@@ -474,6 +494,39 @@ class Prover(_ConstraintSystem):
             return proof.raw[:rc], [V.raw[32 * i:32 * i + 32] for i in range(m)]
         finally:
             self.ctx.lib.bpg_circuit_destroy(circ)
+
+
+def prove_batch(provers, bp_gens, ext_rngs=None, flags=0):
+    """Prover::prove(&bp_gens) of many provers in ONE call (bpg_r1cs_prove_batch) -> list of (proof bytes, [V commitments]),
+    entry i being what provers[i].prove(bp_gens, ext_rngs[i], flags) returns.  The provers share one context; ext_rngs
+    (one 32-byte string per prover) default to os.urandom."""
+    if not provers:
+        return []
+    ctx = provers[0].ctx
+    if any(p.ctx is not ctx for p in provers):
+        raise ValueError("prove_batch: every prover must use the same Context")
+    for p in provers:
+        npad = 1
+        while npad < p.num_vars:
+            npad *= 2
+        if bp_gens.gens_capacity < npad:
+            raise R1CSError("InvalidGeneratorsLength")
+    exts = list(ext_rngs) if ext_rngs is not None else [os.urandom(32) for _ in provers]
+    if len(exts) != len(provers):
+        raise ValueError("prove_batch: %d ext_rngs for %d provers" % (len(exts), len(provers)))
+    enc = lambda xs: b"".join(int(x).to_bytes(32, "little") for x in xs)
+    circs = []
+    try:
+        items = []
+        for p, ext in zip(provers, exts):
+            circs.append(p._circuit(len(p.v)))
+            aL, aR, aO = p.witness_bytes()
+            items.append((circs[-1], p.label, aL, aR, aO, enc(p.v), enc(p.v_blinding), ext))
+        out = ctx.prove_batch(items, flags)
+    finally:
+        for c in circs:
+            ctx.lib.bpg_circuit_destroy(c)
+    return [(proof, [V[32 * i:32 * i + 32] for i in range(len(p.v))]) for (proof, V), p in zip(out, provers)]
 
 
 class Verifier(_ConstraintSystem):

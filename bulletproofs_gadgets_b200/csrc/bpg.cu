@@ -8,6 +8,7 @@
 #include "kernels_core.cuh"
 #include "kernels_msm.cuh"
 #include "kernels_vec.cuh"
+#include "kernels_batch.cuh"
 
 #include <stdio.h>
 #include <stdlib.h>
@@ -992,3 +993,4 @@ extern "C" int bpg_host_rng_draw64(const uint8_t *label, size_t label_len, const
 }
 
 #include "prover.inl"
+#include "prover_batch.inl"

@@ -169,6 +169,26 @@ long bpg_r1cs_prove(bpg_ctx *ctx, bpg_circuit *c, const uint8_t *label, size_t l
  * the hint.  Up to two proofs can be pending; further hints are ignored.  flags as for bpg_r1cs_prove. */
 int bpg_r1cs_prove_prefetch(bpg_ctx *ctx, bpg_circuit *c, const uint8_t *label, size_t label_len, const uint8_t *v,
                             const uint8_t *v_blinding, const uint8_t ext_rng32[32], unsigned flags);
+/* K independent proofs in one call.  Proof i is byte-identical to
+ * bpg_r1cs_prove(ctx, circuits[i], labels[i], label_lens[i], aL[i], aR[i], aO[i], v[i], v_blinding[i],
+ *                ext_rng32 + 32 i, flags, V_out[i], proofs[i], proof_caps[i])
+ * and its length is written to proof_lens[i].  The proofs of padded size N <= 4096 run through the phases of Prover::prove in
+ * lockstep: each phase is one set of launches and one host round trip for all of them (5 + max lg N round trips per pass,
+ * independent of the count); a proof with a larger N is proved by bpg_r1cs_prove inside the call, so any mix may be passed.
+ *  - Every argument of every proof is checked before any device work: a NULL array or entry where bpg_r1cs_prove needs a
+ *    pointer (V_out and its entries may be NULL), proof_caps[i] below the size of proof i or a generator capacity below N_i
+ *    fail the whole call with the code bpg_r1cs_prove returns (BPG_E_ARG / BPG_E_SIZE) for the first such proof; nothing is
+ *    written then and proof_lens is zeroed.  count = 0 returns BPG_OK.
+ *  - flags: 0, BPG_FLAG_LEGACY_FRAMING, BPG_FLAG_NO_LATE_FOLD (a no-op at the batched sizes).  BPG_FLAG_FAST_BLINDING,
+ *    BPG_FLAG_WITNESS_ON_DEVICE, BPG_FLAG_FORCE_LATE_FOLD and a sharded context (world > 1) return BPG_E_ARG.  Witness
+ *    buffers are host pointers.
+ *  - The batched path neither uses nor consumes bpg_r1cs_prove_prefetch hints; a delegated proof behaves as bpg_r1cs_prove.
+ *  - Secrets (witness, s_L / s_R, l / r vectors, blindings) are wiped on the device and on the host before the call returns.
+ *  - count has no upper limit: the batch is split internally into passes of bounded scratch, with unchanged bytes. */
+int bpg_r1cs_prove_batch(bpg_ctx *ctx, size_t count, bpg_circuit *const *circuits, const uint8_t *const *labels,
+                         const size_t *label_lens, const uint8_t *const *aL, const uint8_t *const *aR, const uint8_t *const *aO,
+                         const uint8_t *const *v, const uint8_t *const *v_blinding, const uint8_t *ext_rng32, unsigned flags,
+                         uint8_t *const *V_out, uint8_t *const *proofs, const size_t *proof_caps, size_t *proof_lens);
 /* Verifier::new(label) + commit(V_i)* + (constraints) + verify(&proof,&pc_gens,&bp_gens)  [ext; verifier.rs:51-53,90].
  * *accept = 1 for Ok(()), 0 for Err(VerificationError | FormatError); the return value only reports library errors. */
 int bpg_r1cs_verify(bpg_ctx *ctx, bpg_circuit *c, const uint8_t *label, size_t label_len, const uint8_t *V32,

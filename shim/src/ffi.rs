@@ -61,6 +61,7 @@ extern "C" {
     pub fn bpg_witness_eval(ctx: *mut BpgCtx, n: usize, m: usize, lc_ptr: *const u32, term_var: *const u32, term_coeff: *const u8, v: *const u8, aL: *mut u8, aR: *mut u8, aO: *mut u8) -> i32;
     pub fn bpg_r1cs_prove(ctx: *mut BpgCtx, c: *mut BpgCircuit, label: *const u8, label_len: usize, aL: *const u8, aR: *const u8, aO: *const u8, v: *const u8, v_blinding: *const u8, ext_rng32: *const u8, flags: u32, V_out: *mut u8, proof: *mut u8, proof_cap: usize) -> i64;
     pub fn bpg_r1cs_prove_prefetch(ctx: *mut BpgCtx, c: *mut BpgCircuit, label: *const u8, label_len: usize, v: *const u8, v_blinding: *const u8, ext_rng32: *const u8, flags: u32) -> i32;
+    pub fn bpg_r1cs_prove_batch(ctx: *mut BpgCtx, count: usize, circuits: *const *mut BpgCircuit, labels: *const *const u8, label_lens: *const usize, aL: *const *const u8, aR: *const *const u8, aO: *const *const u8, v: *const *const u8, v_blinding: *const *const u8, ext_rng32: *const u8, flags: u32, V_out: *const *mut u8, proofs: *const *mut u8, proof_caps: *const usize, proof_lens: *mut usize) -> i32;
     pub fn bpg_r1cs_verify(ctx: *mut BpgCtx, c: *mut BpgCircuit, label: *const u8, label_len: usize, V32: *const u8, proof: *const u8, proof_len: usize, ext_rng32: *const u8, flags: u32, accept: *mut i32) -> i32;
     pub fn bpg_r1cs_verify_batch(ctx: *mut BpgCtx, count: usize, circuits: *const *mut BpgCircuit, labels: *const *const u8, label_lens: *const usize, V32: *const *const u8, proofs: *const *const u8, proof_lens: *const usize, ext_rng32: *const u8, flags: u32, accept: *mut i32) -> i32;
     pub fn bpg_transcript_new(label: *const u8, len: usize) -> *mut BpgTranscript;

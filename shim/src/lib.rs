@@ -42,6 +42,17 @@ lazy_static! {
 /// kind 0 = a_L, 1 = a_R, 2 = a_O, 3 = V, 4 = One (r1cs::Variable as recorded by ConstraintSystem::constrain).
 pub struct FlatConstraints { pub row_ptr: Vec<u32>, pub term_var: Vec<u32>, pub term_coeff: Vec<u8> }
 
+/// One statement of Device::r1cs_prove_batch: the arguments of one Device::r1cs_prove call.
+pub struct ProveJob<'a> {
+    pub label: &'a [u8],
+    pub cs: &'a FlatConstraints,
+    pub a_l: &'a [u8],
+    pub a_r: &'a [u8],
+    pub a_o: &'a [u8],
+    pub v: &'a [u8],
+    pub v_blinding: &'a [u8],
+}
+
 pub const VAR_L: u32 = 0;
 pub const VAR_R: u32 = 1;
 pub const VAR_O: u32 = 2;
@@ -138,6 +149,54 @@ impl Device {
         proof.truncate(len as usize);
         vout.truncate(32 * m);
         Ok((proof, vout))
+    }
+    /// Prover::prove for many statements in one call (bpg_r1cs_prove_batch): entry i is what r1cs_prove returns for jobs[i]
+    /// with the same thread_rng bytes.  Small circuits (padded size <= 4096) are proved in lockstep, larger ones one by one.
+    pub fn r1cs_prove_batch(&mut self, jobs: &[ProveJob], flags: u32) -> Result<Vec<(Vec<u8>, Vec<u8>)>, BpgError> {
+        use rand::RngCore;
+        let k = jobs.len();
+        let mut ext = vec![0u8; 32 * k];
+        rand::thread_rng().fill_bytes(&mut ext);
+        let mut circuits: Vec<*mut ffi::BpgCircuit> = Vec::with_capacity(k);
+        for j in jobs {
+            let (n, m) = (j.a_l.len() / 32, j.v.len() / 32);
+            assert!(j.a_r.len() == j.a_l.len() && j.a_o.len() == j.a_l.len() && j.v_blinding.len() == j.v.len());
+            let mut circuit = ptr::null_mut();
+            let rc = unsafe { ffi::bpg_circuit_create(self.ctx, n, m, j.cs.rows(), j.cs.row_ptr.as_ptr(), j.cs.term_var.as_ptr(), j.cs.term_coeff.as_ptr(), &mut circuit) };
+            if rc != ffi::BPG_OK {
+                for c in &circuits { unsafe { ffi::bpg_circuit_destroy(*c) } }
+                return Err(Device::error(self.ctx, rc));
+            }
+            circuits.push(circuit);
+        }
+        let cap = 1 + 32 * (14 + 64 + 2);
+        let mut proofs: Vec<Vec<u8>> = (0..k).map(|_| vec![0u8; cap]).collect();
+        let mut vouts: Vec<Vec<u8>> = jobs.iter().map(|j| vec![0u8; std::cmp::max(j.v.len(), 32)]).collect();
+        let labels: Vec<*const u8> = jobs.iter().map(|j| j.label.as_ptr()).collect();
+        let label_lens: Vec<usize> = jobs.iter().map(|j| j.label.len()).collect();
+        let a_l: Vec<*const u8> = jobs.iter().map(|j| j.a_l.as_ptr()).collect();
+        let a_r: Vec<*const u8> = jobs.iter().map(|j| j.a_r.as_ptr()).collect();
+        let a_o: Vec<*const u8> = jobs.iter().map(|j| j.a_o.as_ptr()).collect();
+        let v: Vec<*const u8> = jobs.iter().map(|j| j.v.as_ptr()).collect();
+        let v_blinding: Vec<*const u8> = jobs.iter().map(|j| j.v_blinding.as_ptr()).collect();
+        let vout_ptrs: Vec<*mut u8> = vouts.iter_mut().map(|x| x.as_mut_ptr()).collect();
+        let proof_ptrs: Vec<*mut u8> = proofs.iter_mut().map(|x| x.as_mut_ptr()).collect();
+        let caps = vec![cap; k];
+        let mut lens = vec![0usize; k];
+        let rc = unsafe {
+            ffi::bpg_r1cs_prove_batch(self.ctx, k, circuits.as_ptr(), labels.as_ptr(), label_lens.as_ptr(), a_l.as_ptr(), a_r.as_ptr(), a_o.as_ptr(),
+                                      v.as_ptr(), v_blinding.as_ptr(), ext.as_ptr(), flags, vout_ptrs.as_ptr(), proof_ptrs.as_ptr(), caps.as_ptr(),
+                                      lens.as_mut_ptr())
+        };
+        for c in &circuits { unsafe { ffi::bpg_circuit_destroy(*c) } }
+        self.check(rc)?;
+        let mut out = Vec::with_capacity(k);
+        for (i, (mut proof, mut vout)) in proofs.into_iter().zip(vouts.into_iter()).enumerate() {
+            proof.truncate(lens[i]);
+            vout.truncate(jobs[i].v.len());
+            out.push((proof, vout));
+        }
+        Ok(out)
     }
     /// Verifier::verify: Ok(true) for Ok(()), Ok(false) for Err(VerificationError | FormatError)
     pub fn r1cs_verify(&mut self, label: &[u8], cs: &FlatConstraints, n: usize, commitments: &[u8], proof: &[u8], flags: u32) -> Result<bool, BpgError> {

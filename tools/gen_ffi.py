@@ -23,6 +23,8 @@ def param(p):
     stars = ty.count("*") + (1 if arr else 0)
     if stars == 2 and const and base == "bpg_circuit":   # bpg_circuit *const *circuits
         return name, "*const *mut BpgCircuit"
+    if stars == 2 and const and base == "uint8_t" and not ty.startswith("const"):  # uint8_t *const *proofs
+        return name, "*const *mut u8"
     if stars == 2 and const and base == "uint8_t":       # const uint8_t *const *labels
         return name, "*const *const u8"
     rt = BASE[base]
