@@ -3,8 +3,9 @@
 //
 // The K proofs of a batch keep their vectors at ragged offsets off_p = sum_{k<p} N_k of shared buffers.  A kernel either
 // walks 128-element blocks of those vectors -- blkp[block] = proof, the element index is (block - blk0_p) * 128 + thread --
-// or looks its proof up by binary search over a prefix held in the descriptors.  Each body is that of the per-proof kernel
-// in kernels_vec.cuh / kernels_msm.cuh, so every scalar and every point equals what bpg_r1cs_prove computes.
+// or looks its proof up by binary search over a prefix held in the descriptors, and hands the per-element body of
+// kernels_vec.cuh / kernels_msm.cuh (the one its per-proof kernel calls) base pointers offset to that proof, so every scalar
+// and every point equals what bpg_r1cs_prove computes.
 #pragma once
 #include "kernels_msm.cuh"
 #include "kernels_vec.cuh"
@@ -34,7 +35,7 @@ __device__ __forceinline__ uint32_t pb_find(const pb_desc *__restrict__ D, uint3
     return lo;
 }
 
-// s_L, s_R of every proof from its raw draws (k_sc_reduce_wide)
+// s_L, s_R of every proof from its raw draws
 __global__ void __launch_bounds__(128) k_pb_reduce_wide(const pb_desc *__restrict__ D, const uint32_t *__restrict__ blkp, const uint32_t *__restrict__ raw,
                                                         sc *__restrict__ sL, sc *__restrict__ sR) {
     const pb_desc &P = D[blkp[blockIdx.x]];
@@ -42,25 +43,18 @@ __global__ void __launch_bounds__(128) k_pb_reduce_wide(const pb_desc *__restric
     if (i >= P.n) return;
 #pragma unroll 1
     for (int side = 0; side < 2; side++) {
-        const uint4 *src = (const uint4 *)(raw + 16ull * (P.roff + side * P.n + i));
-        u32 R[16];
-#pragma unroll
-        for (int k = 0; k < 4; k++) { uint4 q = src[k]; R[4 * k] = q.x; R[4 * k + 1] = q.y; R[4 * k + 2] = q.z; R[4 * k + 3] = q.w; }
         sc r;
-        sc_reduce512(r, R);
+        reduce_wide_draw(r, raw + 16ull * (P.roff + side * P.n + i));
         st_sc(side ? &sR[P.off + i] : &sL[P.off + i], r);
     }
 }
 
-// Power tables sized per proof: base^e = lo[e & 63] * hi[e >> 6] with lo[t] = base^t (t < 64), hi[j] = base^(64 j) -- the same
-// field elements as bpg_r1cs_prove's 1024-entry split, in a few KB per proof (table entries: 64 + (max exponent >> 6) + 2).
-#define PB_POW_LO 64u
-__host__ __device__ __forceinline__ uint32_t pb_pow_entries(uint32_t max_exp) { return PB_POW_LO + (max_exp >> 6) + 2u; }
-__device__ __forceinline__ void pb_pow(sc &r, const sc *__restrict__ tab, uint32_t e) {
-    sc a, b;
-    ld_sc(a, &tab[e & (PB_POW_LO - 1)]);
-    if (e >> 6) { ld_sc(b, &tab[PB_POW_LO + (e >> 6)]); sc_mul(r, a, b); } else r = a;
-}
+// Power tables sized per proof: lo[t] = base^t (t < 64) followed by hi[j] = base^(64 j), read as pow_lookup<PB_POW_LG>(r, tab,
+// tab + PB_POW_LO, e) -- the same field elements as bpg_r1cs_prove's 1024-entry split, in a few KB per proof (table entries:
+// 64 + (max exponent >> 6) + 2)
+#define PB_POW_LG 6
+#define PB_POW_LO (1u << PB_POW_LG)
+__host__ __device__ __forceinline__ uint32_t pb_pow_entries(uint32_t max_exp) { return PB_POW_LO + (max_exp >> PB_POW_LG) + 2u; }
 // z, y, y^-1 tables of every proof, one thread per entry of the concatenated tables (total entries: the last proof's pt + 3 tables)
 __global__ void __launch_bounds__(128) k_pb_pow_tables(const pb_desc *__restrict__ D, uint32_t K, uint32_t total, const sc *__restrict__ small,
                                                        sc *__restrict__ pt) {
@@ -73,7 +67,7 @@ __global__ void __launch_bounds__(128) k_pb_pow_tables(const pb_desc *__restrict
     else { slot = 5u; e -= nz + ny; }               // y^-1
     sc b, r;
     ld_sc(b, &small[PB_SLOTS * p + slot]);
-    sc_pow_u32(r, b, e < PB_POW_LO ? e : (e - PB_POW_LO) << 6);
+    sc_pow_u32(r, b, e < PB_POW_LO ? e : (e - PB_POW_LO) << PB_POW_LG);
     st_sc(&pt[g], r);
 }
 
@@ -82,34 +76,22 @@ __global__ void __launch_bounds__(128) k_pb_flatten_vcols(const pb_desc *__restr
                                                           sc *__restrict__ partial) {
     uint32_t g = blockIdx.x * blockDim.x + threadIdx.x;
     if (g >= nv_total) return;
-    uint32_t p = pb_find(D, K, g, [](const pb_desc &d) { return d.vc0; });
-    const pb_desc &P = D[p];
-    uint32_t c = g - P.vc0;
+    const pb_desc &P = D[pb_find(D, K, g, [](const pb_desc &d) { return d.vc0; })];
+    const uint32_t c = g - P.vc0;
     const sc *zt = pt + P.pt;
-    sc acc; sc_zero(acc);
-    uint32_t k0 = P.vcol_ptr[c], k1 = P.vcol_ptr[c + 1];
-#pragma unroll 1
-    for (uint32_t k = k0; k < k1; k++) {
-        sc zp, cf, q;
-        pb_pow(zp, zt, P.row[k] + 1u);
-        ld_sc(cf, &P.coeff[k]);
-        sc_mul(q, zp, cf);
-        sc_add_r(acc, acc, q);
-    }
+    sc acc;
+    flatten_vcol<PB_POW_LG>(acc, c, P.vcol_ptr, P.row, P.coeff, zt, zt + PB_POW_LO);
     uint32_t d = P.vcol_dst[c];
     if (d & 0x80000000u) st_sc(&partial[P.poff + (d & 0x7FFFFFFFu)], acc); else st_sc(&w[P.woff + d], acc);
 }
 // k_flatten_split: one block per split column of any circuit
 __global__ void __launch_bounds__(128) k_pb_flatten_split(const pb_desc *__restrict__ D, uint32_t K, const sc *__restrict__ partial, sc *__restrict__ w) {
     __shared__ sc smem[128];
-    const uint32_t p = pb_find(D, K, blockIdx.x, [](const pb_desc &d) { return d.sp0; });
-    const uint32_t *sp = D[p].split + 3 * (blockIdx.x - D[p].sp0);
-    const sc *part = partial + D[p].poff + sp[1];
-    const uint32_t cnt = sp[2];
-    sc acc; sc_zero(acc);
-    for (uint32_t k = threadIdx.x; k < cnt; k += 128) { sc x; ld_sc(x, &part[k]); sc_add_r(acc, acc, x); }
-    block_sum_scalars<1>(&acc, smem);
-    if (threadIdx.x == 0) st_sc(&w[D[p].woff + sp[0]], acc);
+    const pb_desc &P = D[pb_find(D, K, blockIdx.x, [](const pb_desc &d) { return d.sp0; })];
+    const uint32_t *sp = P.split + 3 * (blockIdx.x - P.sp0); // (col, first, count)
+    sc acc;
+    block_sum_rows<1>(&acc, partial + P.poff, sp[1], sp[2], smem);
+    if (threadIdx.x == 0) st_sc(&w[P.woff + sp[0]], acc);
 }
 
 // k_poly_phase1, one 128-element block of one proof per block; tparts[block][6]
@@ -118,32 +100,16 @@ __global__ void __launch_bounds__(128) k_pb_poly_phase1(const pb_desc *__restric
                                                         const sc *__restrict__ w, const sc *__restrict__ pt, sc *__restrict__ l1o,
                                                         sc *__restrict__ r0o, sc *__restrict__ r1o, sc *__restrict__ r3o, sc *__restrict__ tparts) {
     __shared__ sc smem[6 * 128];
-    const uint32_t p = blkp[blockIdx.x];
-    const pb_desc &P = D[p];
-    const uint32_t i = (blockIdx.x - P.blk0) * 128u + threadIdx.x, n = P.n;
+    const pb_desc &P = D[blkp[blockIdx.x]];
+    const uint32_t i = (blockIdx.x - P.blk0) * 128u + threadIdx.x;
     sc t[6];
 #pragma unroll
     for (int k = 0; k < 6; k++) sc_zero(t[k]);
-    if (i < n) {
+    if (i < P.n) {
         const sc *yt = pt + P.pt + P.nz, *yit = yt + P.ny;
-        const sc *W = w + P.woff;
-        const uint32_t o = P.off + i;
-        sc yi, yinv, a_l, a_r, a_o, s_l, s_r, wl, wr, wo, l1, r0, r1, r3, q;
-        pb_pow(yi, yt, i);
-        pb_pow(yinv, yit, i);
-        ld_sc(a_l, &aL[o]); ld_sc(a_r, &aR[o]); ld_sc(a_o, &aO[o]); ld_sc(s_l, &sL[o]); ld_sc(s_r, &sR[o]);
-        ld_sc(wl, &W[i]); ld_sc(wr, &W[n + i]); ld_sc(wo, &W[2 * (size_t)n + i]);
-        sc_mul(q, yinv, wr); sc_add_r(l1, a_l, q);
-        sc_sub_r(r0, wo, yi);
-        sc_mul(q, yi, a_r); sc_add_r(r1, q, wl);
-        sc_mul(r3, yi, s_r);
-        st_sc(&l1o[o], l1); st_sc(&r0o[o], r0); st_sc(&r1o[o], r1); st_sc(&r3o[o], r3);
-        sc_mul(q, l1, r0); sc_add_r(t[0], t[0], q);
-        sc_mul(q, l1, r1); sc_add_r(t[1], t[1], q); sc_mul(q, a_o, r0); sc_add_r(t[1], t[1], q);
-        sc_mul(q, a_o, r1); sc_add_r(t[2], t[2], q); sc_mul(q, s_l, r0); sc_add_r(t[2], t[2], q);
-        sc_mul(q, l1, r3); sc_add_r(t[3], t[3], q); sc_mul(q, s_l, r1); sc_add_r(t[3], t[3], q);
-        sc_mul(q, a_o, r3); sc_add_r(t[4], t[4], q);
-        sc_mul(q, s_l, r3); sc_add_r(t[5], t[5], q);
+        const uint32_t o = P.off;
+        poly_phase1_elem<PB_POW_LG>(i, P.n, aL + o, aR + o, aO + o, sL + o, sR + o, w + P.woff, yt, yt + PB_POW_LO, yit, yit + PB_POW_LO, l1o + o,
+                                    r0o + o, r1o + o, r3o + o, t);
     }
     block_sum_scalars<6>(t, smem);
     if (threadIdx.x == 0) {
@@ -156,15 +122,8 @@ __global__ void __launch_bounds__(128) k_pb_phase1_out(const pb_desc *__restrict
                                                        const uint32_t *__restrict__ ooff, sc *__restrict__ out) {
     __shared__ sc smem[6 * 128];
     const pb_desc &P = D[blockIdx.x];
-    const uint32_t nb = (P.N + 127u) / 128u;
     sc acc[6];
-#pragma unroll
-    for (int k = 0; k < 6; k++) sc_zero(acc[k]);
-    for (uint32_t b = threadIdx.x; b < nb; b += 128) {
-#pragma unroll
-        for (int k = 0; k < 6; k++) { sc x; ld_sc(x, &tparts[(size_t)(P.blk0 + b) * 6 + k]); sc_add_r(acc[k], acc[k], x); }
-    }
-    block_sum_scalars<6>(acc, smem);
+    block_sum_rows<6>(acc, tparts, P.blk0, (P.N + 127u) / 128u, smem);
     sc *o = out + ooff[blockIdx.x];
     if (threadIdx.x == 0) {
 #pragma unroll
@@ -182,36 +141,10 @@ __global__ void __launch_bounds__(128) k_pb_poly_phase2(const pb_desc *__restric
     const pb_desc &P = D[p];
     const uint32_t i = (blockIdx.x - P.blk0) * 128u + threadIdx.x;
     if (i >= P.N) return;
-    const sc *xs = small + PB_SLOTS * p + 6;
     const sc *yt = pt + P.pt + P.nz, *yit = yt + P.ny;
-    const uint32_t o = P.off + i;
-    sc x, x2, x3, u, yinv;
-    ld_sc(x, &xs[0]); ld_sc(x2, &xs[1]); ld_sc(x3, &xs[2]); ld_sc(u, &xs[3]);
-    pb_pow(yinv, yit, i);
-    sc one; sc_set_u32(one, 1);
-    if (i < P.n) {
-        sc v, q, acc;
-        ld_sc(v, &l1[o]); sc_mul(acc, x, v);
-        ld_sc(v, &aO[o]); sc_mul(q, x2, v); sc_add_r(acc, acc, q);
-        ld_sc(v, &sL[o]); sc_mul(q, x3, v); sc_add_r(acc, acc, q);
-        st_sc(&a[o], acc);
-        ld_sc(acc, &r0[o]);
-        ld_sc(v, &r1[o]); sc_mul(q, x, v); sc_add_r(acc, acc, q);
-        ld_sc(v, &r3[o]); sc_mul(q, x3, v); sc_add_r(acc, acc, q);
-        st_sc(&b[o], acc);
-        st_sc(&EG[o], one);
-        st_sc(&EH[o], yinv);
-    } else {
-        sc z, yi, ny, eh;
-        sc_zero(z);
-        pb_pow(yi, yt, i);
-        sc_neg_r(ny, yi);
-        st_sc(&a[o], z);
-        st_sc(&b[o], ny);
-        st_sc(&EG[o], u);
-        sc_mul(eh, yinv, u);
-        st_sc(&EH[o], eh);
-    }
+    const uint32_t o = P.off;
+    poly_phase2_elem<PB_POW_LG>(i, P.n, small + PB_SLOTS * p + 6, l1 + o, aO + o, sL + o, r0 + o, r1 + o, r3 + o, yt, yt + PB_POW_LO, yit,
+                                yit + PB_POW_LO, a + o, b + o, EG + o, EH + o);
 }
 
 // ---- inner-product round j: proof p takes part while j < lgN_p (h = N_p >> (j + 1), nj = 2 h)
@@ -224,13 +157,7 @@ __global__ void __launch_bounds__(128) k_pb_ipp_cross(const pb_desc *__restrict_
     const uint32_t i = (blockIdx.x - P.blk0) * 128u + threadIdx.x, h = P.N >> (j + 1);
     sc t[2];
     sc_zero(t[0]); sc_zero(t[1]);
-    if (i < h) {
-        const sc *A = a + P.off, *B = b + P.off;
-        sc al, ah, bl, bh, q;
-        ld_sc(al, &A[i]); ld_sc(ah, &A[h + i]); ld_sc(bl, &B[i]); ld_sc(bh, &B[h + i]);
-        sc_mul(q, al, bh); sc_add_r(t[0], t[0], q);
-        sc_mul(q, ah, bl); sc_add_r(t[1], t[1], q);
-    }
+    if (i < h) ipp_cross_elem(i, h, a + P.off, b + P.off, t);
     block_sum_scalars<2>(t, smem);
     if (threadIdx.x == 0) { st_sc(&cparts[2 * (size_t)blockIdx.x], t[0]); st_sc(&cparts[2 * (size_t)blockIdx.x + 1], t[1]); }
 }
@@ -239,14 +166,8 @@ __global__ void __launch_bounds__(128) k_pb_ipp_cw(const pb_desc *__restrict__ D
     __shared__ sc smem[2 * 128];
     const pb_desc &P = D[blockIdx.x];
     if (j >= P.lgN) return;
-    const uint32_t nb = ((P.N >> (j + 1)) + 127u) / 128u;
     sc acc[2];
-    sc_zero(acc[0]); sc_zero(acc[1]);
-    for (uint32_t k = threadIdx.x; k < nb; k += 128) {
-#pragma unroll
-        for (int s = 0; s < 2; s++) { sc x; ld_sc(x, &cparts[2 * (size_t)(P.blk0 + k) + s]); sc_add_r(acc[s], acc[s], x); }
-    }
-    block_sum_scalars<2>(acc, smem);
+    block_sum_rows<2>(acc, cparts, P.blk0, ((P.N >> (j + 1)) + 127u) / 128u, smem);
     if (threadIdx.x == 0) {
         sc *sm = small + PB_SLOTS * blockIdx.x;
         sc w, r;
@@ -262,12 +183,8 @@ __global__ void __launch_bounds__(128) k_pb_ipp_expand(const pb_desc *__restrict
     const pb_desc &P = D[blkp[blockIdx.x]];
     const uint32_t i = (blockIdx.x - P.blk0) * 128u + threadIdx.x;
     if (j >= P.lgN || i >= P.N) return;
-    const uint32_t nj = P.N >> j, h = nj >> 1, r = i & (nj - 1);
-    const uint32_t src = P.off + (r >= h ? r - h : r + h), o = P.off + i;
-    sc av, bv, eg, eh, q;
-    ld_sc(av, &a[src]); ld_sc(bv, &b[src]); ld_sc(eg, &EG[o]); ld_sc(eh, &EH[o]);
-    sc_mul(q, av, eg); st_sc(&sG[o], q);
-    sc_mul(q, bv, eh); st_sc(&sH[o], q);
+    const uint32_t o = P.off;
+    ipp_expand_elem(i, P.N >> j, a + o, b + o, EG + o, EH + o, sG + o, sH + o);
 }
 // k_ipp_fold of every active proof; uu[2 p], uu[2 p + 1] = u_j, u_j^-1 of proof p
 __global__ void __launch_bounds__(128) k_pb_ipp_fold(const pb_desc *__restrict__ D, const uint32_t *__restrict__ blkp, uint32_t j, const sc *__restrict__ uu,
@@ -276,20 +193,11 @@ __global__ void __launch_bounds__(128) k_pb_ipp_fold(const pb_desc *__restrict__
     const pb_desc &P = D[p];
     const uint32_t i = (blockIdx.x - P.blk0) * 128u + threadIdx.x;
     if (j >= P.lgN || i >= P.N) return;
-    const uint32_t nj = P.N >> j, h = nj >> 1, o = P.off + i;
-    sc u, ui, e, q;
+    const uint32_t nj = P.N >> j, h = nj >> 1, o = P.off;
+    sc u, ui;
     ld_sc(u, &uu[2 * p]); ld_sc(ui, &uu[2 * p + 1]);
-    const bool right = (i & (nj - 1)) >= h;
-    ld_sc(e, &EG[o]); sc_mul(q, e, right ? u : ui); st_sc(&EG[o], q);
-    ld_sc(e, &EH[o]); sc_mul(q, e, right ? ui : u); st_sc(&EH[o], q);
-    if (i < h) {
-        sc lo, hi, r;
-        sc *A = a + P.off, *B = b + P.off;
-        ld_sc(lo, &A[i]); ld_sc(hi, &A[h + i]);
-        sc_mul(q, lo, u); sc_mul(r, hi, ui); sc_add_r(q, q, r); st_sc(&A[i], q);
-        ld_sc(lo, &B[i]); ld_sc(hi, &B[h + i]);
-        sc_mul(q, lo, ui); sc_mul(r, hi, u); sc_add_r(q, q, r); st_sc(&B[i], q);
-    }
+    ipp_fold_factors(i, nj, h, u, ui, EG + o, EH + o);
+    if (i < h) ipp_fold_ab(i, h, u, ui, a + o, b + o);
 }
 // final (a, b) of every proof -> out[2 p], out[2 p + 1]
 __global__ void __launch_bounds__(128) k_pb_final_ab(const pb_desc *__restrict__ D, uint32_t K, const sc *__restrict__ a, const sc *__restrict__ b,
@@ -317,27 +225,11 @@ __global__ void __launch_bounds__(256) k_many_digits(const msm_seg *__restrict__
         while (hi - lo > 1) { uint32_t mid = (lo + hi) >> 1; if (segs[mid].start <= t) lo = mid; else hi = mid; }
         const msm_seg S = segs[lo];
         uint32_t j = t - S.start;
-        sc k;
-        ld_sc(k, &S.scalars[j]);
-        if (S.reduce) sc_reduce(k, k);
-        sc_digits16(d, k);
+        msm_seg_digits(S, j, d, pidx);
         grp = S.group;
         if (S.alt) grp ^= ((j + S.j0) >> (S.alt - 1)) & 1u;
-        pidx = S.p0 + j;
     }
     const uint32_t base = grp * 2u * BPG_MAT_NB;
 #pragma unroll
-    for (int w = 0; w < 16; w++) {
-        int dw = d[w];
-        uint32_t ent = (uint32_t)w * ptotal + pidx;
-        int dl = ((dw + 128) & 255) - 128; // [-128, 127]
-        int dh = (dw - dl) >> 8;           // exact ; [-128, 128]
-#pragma unroll
-        for (int part = 0; part < 2; part++) {
-            int dd = part ? dh : dl;
-            uint32_t mag = dd < 0 ? (uint32_t)(-dd) : (uint32_t)dd;
-            uint32_t pos = warp_counter_add(counts_or_cursor, base + part * BPG_MAT_NB + mag, dd != 0);
-            if (SCATTER && dd != 0) sorted[pos] = ent | (dd < 0 ? 0x80000000u : 0u);
-        }
-    }
+    for (int w = 0; w < 16; w++) emit_split_digit<SCATTER>(counts_or_cursor, sorted, base, d[w], (uint32_t)w * ptotal + pidx);
 }

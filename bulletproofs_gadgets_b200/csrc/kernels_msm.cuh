@@ -62,6 +62,19 @@ __device__ __forceinline__ uint32_t warp_counter_add(uint32_t *__restrict__ arr,
     }
     return active ? atomicAdd(&arr[bkt], 1u) : 0u;
 }
+// SPLIT = 1 pairs of one digit dw = dl + 256 dh: buckets base + |dl| and base + 129 + |dh|, entry ent with the digit's sign
+template <int SCATTER>
+__device__ __forceinline__ void emit_split_digit(uint32_t *__restrict__ counts_or_cursor, uint32_t *__restrict__ sorted, uint32_t base, int dw, uint32_t ent) {
+    int dl = ((dw + 128) & 255) - 128; // [-128, 127]
+    int dh = (dw - dl) >> 8;           // exact ; [-128, 128]
+#pragma unroll
+    for (int part = 0; part < 2; part++) {
+        int dd = part ? dh : dl;
+        uint32_t mag = dd < 0 ? (uint32_t)(-dd) : (uint32_t)dd;
+        uint32_t pos = warp_counter_add(counts_or_cursor, base + part * 129u + mag, dd != 0);
+        if (SCATTER && dd != 0) sorted[pos] = ent | (dd < 0 ? 0x80000000u : 0u);
+    }
+}
 template <int SCATTER, int SPLIT>
 __global__ void __launch_bounds__(256) k_msm_digits(msm_params P, uint32_t *__restrict__ counts_or_cursor, uint32_t *__restrict__ sorted) {
     uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
@@ -94,15 +107,7 @@ __global__ void __launch_bounds__(256) k_msm_digits(msm_params P, uint32_t *__re
         uint32_t ent = P.varbase ? pidx : (uint32_t)w * P.ptotal + pidx;
         if (P.varbase) base = (grp + (uint32_t)w) * gstride;
         if (SPLIT) {
-            int dl = ((dw + 128) & 255) - 128; // [-128, 127]
-            int dh = (dw - dl) >> 8;           // exact ; [-128, 128]
-#pragma unroll
-            for (int part = 0; part < 2; part++) {
-                int dd = part ? dh : dl;
-                uint32_t mag = dd < 0 ? (uint32_t)(-dd) : (uint32_t)dd;
-                uint32_t pos = warp_counter_add(counts_or_cursor, base + part * 129u + mag, dd != 0);
-                if (SCATTER && dd != 0) sorted[pos] = ent | (dd < 0 ? 0x80000000u : 0u);
-            }
+            emit_split_digit<SCATTER>(counts_or_cursor, sorted, base, dw, ent);
         } else {
             uint32_t mag = dw < 0 ? (uint32_t)(-dw) : (uint32_t)dw;
             uint32_t pos = warp_counter_add(counts_or_cursor, base + mag, dw != 0);

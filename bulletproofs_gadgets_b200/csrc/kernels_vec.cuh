@@ -47,11 +47,13 @@ __device__ __forceinline__ void sc_zero(sc &r) {
 #pragma unroll
     for (int i = 0; i < 8; i++) r.v[i] = 0;
 }
-// base^e from the two-level tables lo[e & 1023] * hi[e >> 10]
+// base^e from the two-level tables lo[e & (2^LO - 1)] * hi[e >> LO]  (lo[t] = base^t, hi[j] = base^(2^LO j)).
+// bpg_r1cs_prove uses LO = 10; the batch prover LO = 6 (tables sized per proof, kernels_batch.cuh).
+template <int LO>
 __device__ __forceinline__ void pow_lookup(sc &r, const sc *__restrict__ lo, const sc *__restrict__ hi, uint32_t e) {
     sc a, b;
-    ld_sc(a, &lo[e & 1023u]);
-    if (e >> 10) { ld_sc(b, &hi[e >> 10]); sc_mul(r, a, b); } else r = a;
+    ld_sc(a, &lo[e & ((1u << LO) - 1u)]);
+    if (e >> LO) { ld_sc(b, &hi[e >> LO]); sc_mul(r, a, b); } else r = a;
 }
 // block-wide sum of NS scalars per thread (blockDim.x == 128); result valid in thread 0
 template <int NS>
@@ -78,21 +80,38 @@ __device__ __forceinline__ void block_sum_scalars(sc *vals, sc *smem /* [NS][128
     }
 }
 
+// zero NS accumulators, add the rows first + threadIdx.x, first + threadIdx.x + 128, ... < first + cnt of rows (row-major
+// [][NS]) into them and sum them over the block (blockDim.x == 128); result valid in thread 0
+template <int NS>
+__device__ __forceinline__ void block_sum_rows(sc *acc, const sc *__restrict__ rows, uint32_t first, uint32_t cnt, sc *smem /* [NS][128] */) {
+#pragma unroll
+    for (int k = 0; k < NS; k++) sc_zero(acc[k]);
+    for (uint32_t p = threadIdx.x; p < cnt; p += 128) {
+#pragma unroll
+        for (int k = 0; k < NS; k++) { sc x; ld_sc(x, &rows[(size_t)(first + p) * NS + k]); sc_add_r(acc[k], acc[k], x); }
+    }
+    block_sum_scalars<NS>(acc, smem);
+}
+
 __global__ void __launch_bounds__(256) k_sc_reduce_inplace(sc *v, uint32_t n) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     sc x; ld_sc(x, &v[i]); sc_reduce(x, x); st_sc(&v[i], x);
 }
-// Scalar::from_bytes_mod_order_wide over raw 64-byte TranscriptRng draws: element i < n goes to outL[i], n <= i < 2n to outR[i - n]
-__global__ void __launch_bounds__(128) k_sc_reduce_wide(const uint32_t *__restrict__ raw, uint32_t n, sc *__restrict__ outL, sc *__restrict__ outR) {
-    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= 2 * n) return;
-    const uint4 *src = (const uint4 *)(raw + 16ull * i);
+// Scalar::from_bytes_mod_order_wide of one raw 64-byte TranscriptRng draw
+__device__ __forceinline__ void reduce_wide_draw(sc &r, const uint32_t *__restrict__ raw) {
+    const uint4 *src = (const uint4 *)raw;
     u32 R[16];
 #pragma unroll
     for (int k = 0; k < 4; k++) { uint4 q = src[k]; R[4 * k] = q.x; R[4 * k + 1] = q.y; R[4 * k + 2] = q.z; R[4 * k + 3] = q.w; }
-    sc r;
     sc_reduce512(r, R);
+}
+// element i < n of the raw draws goes to outL[i], n <= i < 2n to outR[i - n]
+__global__ void __launch_bounds__(128) k_sc_reduce_wide(const uint32_t *__restrict__ raw, uint32_t n, sc *__restrict__ outL, sc *__restrict__ outR) {
+    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= 2 * n) return;
+    sc r;
+    reduce_wide_draw(r, raw + 16ull * i);
     st_sc(i < n ? &outL[i] : &outR[i - n], r);
 }
 // lo[t] = base^t (t < 1024), hi[j] = base^(1024 j) (j < nhi)
@@ -109,13 +128,7 @@ template <int NS>
 __global__ void __launch_bounds__(128) k_sum_partials(const sc *__restrict__ parts, uint32_t nparts, sc *__restrict__ out) {
     __shared__ sc smem[NS * 128];
     sc acc[NS];
-#pragma unroll
-    for (int k = 0; k < NS; k++) sc_zero(acc[k]);
-    for (uint32_t p = threadIdx.x; p < nparts; p += 128) {
-#pragma unroll
-        for (int k = 0; k < NS; k++) { sc x; ld_sc(x, &parts[(size_t)p * NS + k]); sc_add_r(acc[k], acc[k], x); }
-    }
-    block_sum_scalars<NS>(acc, smem);
+    block_sum_rows<NS>(acc, parts, 0, nparts, smem);
     if (threadIdx.x == 0) {
 #pragma unroll
         for (int k = 0; k < NS; k++) st_sc(&out[k], acc[k]);
@@ -126,21 +139,27 @@ __global__ void __launch_bounds__(128) k_sum_partials(const sc *__restrict__ par
 // Entries are sorted by (virtual) column.  A virtual column is a run of <= 32 entries of one variable; it either
 // writes w[dst] directly or, for variables split over several virtual columns, a partial slot (dst | 1<<31).
 // value = sum_k z^(row_k+1) * coeff_k   (coefficients of V / One columns are stored negated).
+template <int LO>
+__device__ __forceinline__ void flatten_vcol(sc &acc, uint32_t c, const uint32_t *__restrict__ vcol_ptr, const uint32_t *__restrict__ e_row,
+                                             const sc *__restrict__ e_coeff, const sc *__restrict__ zlo, const sc *__restrict__ zhi) {
+    sc_zero(acc);
+    uint32_t k0 = vcol_ptr[c], k1 = vcol_ptr[c + 1];
+#pragma unroll 1
+    for (uint32_t k = k0; k < k1; k++) {
+        sc zp, cf, p;
+        pow_lookup<LO>(zp, zlo, zhi, e_row[k] + 1u);
+        ld_sc(cf, &e_coeff[k]);
+        sc_mul(p, zp, cf);
+        sc_add_r(acc, acc, p);
+    }
+}
 __global__ void __launch_bounds__(128) k_flatten_vcols(const uint32_t *__restrict__ vcol_ptr, const uint32_t *__restrict__ vcol_dst, uint32_t nv,
                                                         const uint32_t *__restrict__ e_row, const sc *__restrict__ e_coeff,
                                                         const sc *__restrict__ zlo, const sc *__restrict__ zhi, sc *__restrict__ w, sc *__restrict__ partial) {
     uint32_t c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= nv) return;
-    sc acc; sc_zero(acc);
-    uint32_t k0 = vcol_ptr[c], k1 = vcol_ptr[c + 1];
-#pragma unroll 1
-    for (uint32_t k = k0; k < k1; k++) {
-        sc zp, cf, p;
-        pow_lookup(zp, zlo, zhi, e_row[k] + 1u);
-        ld_sc(cf, &e_coeff[k]);
-        sc_mul(p, zp, cf);
-        sc_add_r(acc, acc, p);
-    }
+    sc acc;
+    flatten_vcol<10>(acc, c, vcol_ptr, e_row, e_coeff, zlo, zhi);
     uint32_t d = vcol_dst[c];
     if (d & 0x80000000u) st_sc(&partial[d & 0x7FFFFFFFu], acc); else st_sc(&w[d], acc);
 }
@@ -151,9 +170,8 @@ __global__ void __launch_bounds__(128) k_flatten_split(const uint32_t *__restric
     uint32_t s = blockIdx.x;
     if (s >= ns) return;
     uint32_t col = split[3 * s], first = split[3 * s + 1], cnt = split[3 * s + 2];
-    sc acc; sc_zero(acc);
-    for (uint32_t k = threadIdx.x; k < cnt; k += 128) { sc x; ld_sc(x, &partial[first + k]); sc_add_r(acc, acc, x); }
-    block_sum_scalars<1>(&acc, smem);
+    sc acc;
+    block_sum_rows<1>(&acc, partial, first, cnt, smem);
     if (threadIdx.x == 0) st_sc(&w[col], acc);
 }
 
@@ -161,6 +179,29 @@ __global__ void __launch_bounds__(128) k_flatten_split(const uint32_t *__restric
 // l1 = aL + y^-i wR ; l2 = aO ; l3 = sL ; r0 = wO - y^i ; r1 = y^i aR + wL ; r3 = y^i sR
 // t1=<l1,r0> t2=<l1,r1>+<l2,r0> t3=<l2,r1>+<l3,r0> t4=<l1,r3>+<l3,r1> t5=<l2,r3> t6=<l3,r3>
 // stores l1,r0,r1,r3 and per-block partial sums of t1..t6.
+template <int LO>
+__device__ __forceinline__ void poly_phase1_elem(uint32_t i, uint32_t n, const sc *__restrict__ aL, const sc *__restrict__ aR, const sc *__restrict__ aO,
+                                                 const sc *__restrict__ sL, const sc *__restrict__ sR, const sc *__restrict__ w /* wL|wR|wO */,
+                                                 const sc *__restrict__ ylo, const sc *__restrict__ yhi, const sc *__restrict__ yilo,
+                                                 const sc *__restrict__ yihi, sc *__restrict__ l1o, sc *__restrict__ r0o, sc *__restrict__ r1o,
+                                                 sc *__restrict__ r3o, sc *t /* [6] */) {
+    sc yi, yinv, a_l, a_r, a_o, s_l, s_r, wl, wr, wo, l1, r0, r1, r3, p;
+    pow_lookup<LO>(yi, ylo, yhi, i);
+    pow_lookup<LO>(yinv, yilo, yihi, i);
+    ld_sc(a_l, &aL[i]); ld_sc(a_r, &aR[i]); ld_sc(a_o, &aO[i]); ld_sc(s_l, &sL[i]); ld_sc(s_r, &sR[i]);
+    ld_sc(wl, &w[i]); ld_sc(wr, &w[n + i]); ld_sc(wo, &w[2 * (size_t)n + i]);
+    sc_mul(p, yinv, wr); sc_add_r(l1, a_l, p);
+    sc_sub_r(r0, wo, yi);
+    sc_mul(p, yi, a_r); sc_add_r(r1, p, wl);
+    sc_mul(r3, yi, s_r);
+    st_sc(&l1o[i], l1); st_sc(&r0o[i], r0); st_sc(&r1o[i], r1); st_sc(&r3o[i], r3);
+    sc_mul(p, l1, r0); sc_add_r(t[0], t[0], p);
+    sc_mul(p, l1, r1); sc_add_r(t[1], t[1], p); sc_mul(p, a_o, r0); sc_add_r(t[1], t[1], p);
+    sc_mul(p, a_o, r1); sc_add_r(t[2], t[2], p); sc_mul(p, s_l, r0); sc_add_r(t[2], t[2], p);
+    sc_mul(p, l1, r3); sc_add_r(t[3], t[3], p); sc_mul(p, s_l, r1); sc_add_r(t[3], t[3], p);
+    sc_mul(p, a_o, r3); sc_add_r(t[4], t[4], p);
+    sc_mul(p, s_l, r3); sc_add_r(t[5], t[5], p);
+}
 __global__ void __launch_bounds__(128) k_poly_phase1(uint32_t n, const sc *__restrict__ aL, const sc *__restrict__ aR, const sc *__restrict__ aO,
                                                       const sc *__restrict__ sL, const sc *__restrict__ sR, const sc *__restrict__ w /* wL|wR|wO */,
                                                       const sc *__restrict__ ylo, const sc *__restrict__ yhi, const sc *__restrict__ yilo,
@@ -170,24 +211,8 @@ __global__ void __launch_bounds__(128) k_poly_phase1(uint32_t n, const sc *__res
     sc t[6];
 #pragma unroll
     for (int k = 0; k < 6; k++) sc_zero(t[k]);
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        sc yi, yinv, a_l, a_r, a_o, s_l, s_r, wl, wr, wo, l1, r0, r1, r3, p;
-        pow_lookup(yi, ylo, yhi, i);
-        pow_lookup(yinv, yilo, yihi, i);
-        ld_sc(a_l, &aL[i]); ld_sc(a_r, &aR[i]); ld_sc(a_o, &aO[i]); ld_sc(s_l, &sL[i]); ld_sc(s_r, &sR[i]);
-        ld_sc(wl, &w[i]); ld_sc(wr, &w[n + i]); ld_sc(wo, &w[2 * (size_t)n + i]);
-        sc_mul(p, yinv, wr); sc_add_r(l1, a_l, p);
-        sc_sub_r(r0, wo, yi);
-        sc_mul(p, yi, a_r); sc_add_r(r1, p, wl);
-        sc_mul(r3, yi, s_r);
-        st_sc(&l1o[i], l1); st_sc(&r0o[i], r0); st_sc(&r1o[i], r1); st_sc(&r3o[i], r3);
-        sc_mul(p, l1, r0); sc_add_r(t[0], t[0], p);
-        sc_mul(p, l1, r1); sc_add_r(t[1], t[1], p); sc_mul(p, a_o, r0); sc_add_r(t[1], t[1], p);
-        sc_mul(p, a_o, r1); sc_add_r(t[2], t[2], p); sc_mul(p, s_l, r0); sc_add_r(t[2], t[2], p);
-        sc_mul(p, l1, r3); sc_add_r(t[3], t[3], p); sc_mul(p, s_l, r1); sc_add_r(t[3], t[3], p);
-        sc_mul(p, a_o, r3); sc_add_r(t[4], t[4], p);
-        sc_mul(p, s_l, r3); sc_add_r(t[5], t[5], p);
-    }
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+        poly_phase1_elem<10>(i, n, aL, aR, aO, sL, sR, w, ylo, yhi, yilo, yihi, l1o, r0o, r1o, r3o, t);
     block_sum_scalars<6>(t, smem);
     if (threadIdx.x == 0) {
 #pragma unroll
@@ -197,15 +222,14 @@ __global__ void __launch_bounds__(128) k_poly_phase1(uint32_t n, const sc *__res
 // l = x l1 + x^2 l2 + x^3 l3 ; r = r0 + x r1 + x^3 r3 ; padding: l = 0, r = -y^i.
 // Also initialises the per-generator IPP factors EG = G_factors, EH = H_factors (1 or u, times y^-i for H).
 // xs = [x, x^2, x^3, u]
-__global__ void __launch_bounds__(128) k_poly_phase2(uint32_t n, uint32_t N, const sc *__restrict__ xs, const sc *__restrict__ l1, const sc *__restrict__ aO,
-                                                      const sc *__restrict__ sL, const sc *__restrict__ r0, const sc *__restrict__ r1, const sc *__restrict__ r3,
-                                                      const sc *__restrict__ ylo, const sc *__restrict__ yhi, const sc *__restrict__ yilo,
-                                                      const sc *__restrict__ yihi, sc *__restrict__ a, sc *__restrict__ b, sc *__restrict__ EG, sc *__restrict__ EH) {
-    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= N) return;
+template <int LO>
+__device__ __forceinline__ void poly_phase2_elem(uint32_t i, uint32_t n, const sc *__restrict__ xs, const sc *__restrict__ l1, const sc *__restrict__ aO,
+                                                 const sc *__restrict__ sL, const sc *__restrict__ r0, const sc *__restrict__ r1, const sc *__restrict__ r3,
+                                                 const sc *__restrict__ ylo, const sc *__restrict__ yhi, const sc *__restrict__ yilo,
+                                                 const sc *__restrict__ yihi, sc *__restrict__ a, sc *__restrict__ b, sc *__restrict__ EG, sc *__restrict__ EH) {
     sc x, x2, x3, u, yinv;
     ld_sc(x, &xs[0]); ld_sc(x2, &xs[1]); ld_sc(x3, &xs[2]); ld_sc(u, &xs[3]);
-    pow_lookup(yinv, yilo, yihi, i);
+    pow_lookup<LO>(yinv, yilo, yihi, i);
     sc one; sc_set_u32(one, 1);
     if (i < n) {
         sc v, p, acc;
@@ -222,7 +246,7 @@ __global__ void __launch_bounds__(128) k_poly_phase2(uint32_t n, uint32_t N, con
     } else {
         sc z, yi, ny, eh;
         sc_zero(z);
-        pow_lookup(yi, ylo, yhi, i);
+        pow_lookup<LO>(yi, ylo, yhi, i);
         sc_neg_r(ny, yi);
         st_sc(&a[i], z);
         st_sc(&b[i], ny);
@@ -231,19 +255,28 @@ __global__ void __launch_bounds__(128) k_poly_phase2(uint32_t n, uint32_t N, con
         st_sc(&EH[i], eh);
     }
 }
+__global__ void __launch_bounds__(128) k_poly_phase2(uint32_t n, uint32_t N, const sc *__restrict__ xs, const sc *__restrict__ l1, const sc *__restrict__ aO,
+                                                      const sc *__restrict__ sL, const sc *__restrict__ r0, const sc *__restrict__ r1, const sc *__restrict__ r3,
+                                                      const sc *__restrict__ ylo, const sc *__restrict__ yhi, const sc *__restrict__ yilo,
+                                                      const sc *__restrict__ yihi, sc *__restrict__ a, sc *__restrict__ b, sc *__restrict__ EG, sc *__restrict__ EH) {
+    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= N) return;
+    poly_phase2_elem<10>(i, n, xs, l1, aO, sL, r0, r1, r3, ylo, yhi, yilo, yihi, a, b, EG, EH);
+}
 
 // ---------------------------------------------------------------- inner-product argument rounds (a6 / a7)
 // current vectors a,b have length nj = 2h.  cparts[block] = (<a_lo,b_hi>, <a_hi,b_lo>)
+__device__ __forceinline__ void ipp_cross_elem(uint32_t i, uint32_t h, const sc *__restrict__ a, const sc *__restrict__ b, sc *t /* [2] */) {
+    sc al, ah, bl, bh, p;
+    ld_sc(al, &a[i]); ld_sc(ah, &a[h + i]); ld_sc(bl, &b[i]); ld_sc(bh, &b[h + i]);
+    sc_mul(p, al, bh); sc_add_r(t[0], t[0], p);
+    sc_mul(p, ah, bl); sc_add_r(t[1], t[1], p);
+}
 __global__ void __launch_bounds__(128) k_ipp_cross(uint32_t h, const sc *__restrict__ a, const sc *__restrict__ b, sc *__restrict__ cparts) {
     __shared__ sc smem[2 * 128];
     sc t[2];
     sc_zero(t[0]); sc_zero(t[1]);
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < h; i += gridDim.x * blockDim.x) {
-        sc al, ah, bl, bh, p;
-        ld_sc(al, &a[i]); ld_sc(ah, &a[h + i]); ld_sc(bl, &b[i]); ld_sc(bh, &b[h + i]);
-        sc_mul(p, al, bh); sc_add_r(t[0], t[0], p);
-        sc_mul(p, ah, bl); sc_add_r(t[1], t[1], p);
-    }
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < h; i += gridDim.x * blockDim.x) ipp_cross_elem(i, h, a, b, t);
     block_sum_scalars<2>(t, smem);
     if (threadIdx.x == 0) { st_sc(&cparts[2 * (size_t)blockIdx.x], t[0]); st_sc(&cparts[2 * (size_t)blockIdx.x + 1], t[1]); }
 }
@@ -259,10 +292,8 @@ __global__ void k_ipp_cw(const sc *__restrict__ c2, const sc *__restrict__ w, sc
 // with r = i mod nj:  r >= h:  G_i -> L with a[r-h]*EG[i],  H_i -> R with b[r-h]*EH[i]
 //                     r <  h:  G_i -> R with a[h+r]*EG[i],  H_i -> L with b[h+r]*EH[i]
 // [i0, i1): the part of [0, N) this call has to produce (a rank of a sharded proof only needs the scalars of its own point range)
-__global__ void __launch_bounds__(128) k_ipp_expand(uint32_t N, uint32_t nj, const sc *__restrict__ a, const sc *__restrict__ b, const sc *__restrict__ EG,
-                                                     const sc *__restrict__ EH, sc *__restrict__ sG, sc *__restrict__ sH, uint32_t i0, uint32_t i1) {
-    uint32_t i = i0 + blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= i1 || i >= N) return;
+__device__ __forceinline__ void ipp_expand_elem(uint32_t i, uint32_t nj, const sc *__restrict__ a, const sc *__restrict__ b, const sc *__restrict__ EG,
+                                                const sc *__restrict__ EH, sc *__restrict__ sG, sc *__restrict__ sH) {
     uint32_t h = nj >> 1, r = i & (nj - 1);
     uint32_t src = r >= h ? r - h : r + h;
     sc av, bv, eg, eh, p;
@@ -270,8 +301,28 @@ __global__ void __launch_bounds__(128) k_ipp_expand(uint32_t N, uint32_t nj, con
     sc_mul(p, av, eg); st_sc(&sG[i], p);
     sc_mul(p, bv, eh); st_sc(&sH[i], p);
 }
+__global__ void __launch_bounds__(128) k_ipp_expand(uint32_t N, uint32_t nj, const sc *__restrict__ a, const sc *__restrict__ b, const sc *__restrict__ EG,
+                                                     const sc *__restrict__ EH, sc *__restrict__ sG, sc *__restrict__ sH, uint32_t i0, uint32_t i1) {
+    uint32_t i = i0 + blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= i1 || i >= N) return;
+    ipp_expand_elem(i, nj, a, b, EG, EH, sG, sH);
+}
 // a' = a_lo u + a_hi u^-1 ; b' = b_lo u^-1 + b_hi u ; EG[i] *= (right half ? u : u^-1) ; EH[i] *= (right half ? u^-1 : u)
 // uu = [u, u^-1].  The per-generator factors are only updated on [i0, i1) (see k_ipp_expand); a, b always in full.
+__device__ __forceinline__ void ipp_fold_factors(uint32_t i, uint32_t nj, uint32_t h, const sc &u, const sc &ui, sc *__restrict__ EG, sc *__restrict__ EH) {
+    sc e, p;
+    bool right = (i & (nj - 1)) >= h;
+    ld_sc(e, &EG[i]); sc_mul(p, e, right ? u : ui); st_sc(&EG[i], p);
+    ld_sc(e, &EH[i]); sc_mul(p, e, right ? ui : u); st_sc(&EH[i], p);
+}
+// (i < h)
+__device__ __forceinline__ void ipp_fold_ab(uint32_t i, uint32_t h, const sc &u, const sc &ui, sc *__restrict__ a, sc *__restrict__ b) {
+    sc lo, hi, p, q;
+    ld_sc(lo, &a[i]); ld_sc(hi, &a[h + i]);
+    sc_mul(p, lo, u); sc_mul(q, hi, ui); sc_add_r(p, p, q); st_sc(&a[i], p);
+    ld_sc(lo, &b[i]); ld_sc(hi, &b[h + i]);
+    sc_mul(p, lo, ui); sc_mul(q, hi, u); sc_add_r(p, p, q); st_sc(&b[i], p);
+}
 __global__ void __launch_bounds__(128) k_ipp_fold(uint32_t N, uint32_t nj, const sc *__restrict__ uu, sc *__restrict__ a, sc *__restrict__ b, sc *__restrict__ EG,
                                                    sc *__restrict__ EH, uint32_t i0, uint32_t i1) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -279,19 +330,8 @@ __global__ void __launch_bounds__(128) k_ipp_fold(uint32_t N, uint32_t nj, const
     uint32_t h = nj >> 1;
     sc u, ui;
     ld_sc(u, &uu[0]); ld_sc(ui, &uu[1]);
-    sc e, p;
-    if (i >= i0 && i < i1) {
-        bool right = (i & (nj - 1)) >= h;
-        ld_sc(e, &EG[i]); sc_mul(p, e, right ? u : ui); st_sc(&EG[i], p);
-        ld_sc(e, &EH[i]); sc_mul(p, e, right ? ui : u); st_sc(&EH[i], p);
-    }
-    if (i < h) {
-        sc lo, hi, q;
-        ld_sc(lo, &a[i]); ld_sc(hi, &a[h + i]);
-        sc_mul(p, lo, u); sc_mul(q, hi, ui); sc_add_r(p, p, q); st_sc(&a[i], p);
-        ld_sc(lo, &b[i]); ld_sc(hi, &b[h + i]);
-        sc_mul(p, lo, ui); sc_mul(q, hi, u); sc_add_r(p, p, q); st_sc(&b[i], p);
-    }
+    if (i >= i0 && i < i1) ipp_fold_factors(i, nj, h, u, ui, EG, EH);
+    if (i < h) ipp_fold_ab(i, h, u, ui, a, b);
 }
 
 // ---------------------------------------------------------------- verifier scalars (a8)
@@ -326,9 +366,9 @@ __global__ void __launch_bounds__(128) k_verify_scalars(uint32_t n, uint32_t N, 
     sc_set_u32(one, 1);
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < N; i += gridDim.x * blockDim.x) {
         sc yinv, s_i, s_r, p, q, gv, hv;
-        pow_lookup(yinv, yilo, yihi, i);
-        pow_lookup(s_i, slo, shi, i);
-        pow_lookup(s_r, slo, shi, N - 1 - i);
+        pow_lookup<10>(yinv, yilo, yihi, i);
+        pow_lookup<10>(s_i, slo, shi, i);
+        pow_lookup<10>(s_r, slo, shi, N - 1 - i);
         sc_mul(p, ia, s_i);
         sc_mul(q, ib, s_r);
         if (i < n) {
