@@ -49,7 +49,11 @@ SYMBOLS = {
     "bpg_mimc_sponge_batch": (_i32, [_vp, _u8p, _u32p, _sz, _u8p, _u8p]),
     "bpg_circuit_create": (_i32, [_vp, _sz, _sz, _sz, _u32p, _u32p, _u8p, C.POINTER(_vp)]),
     "bpg_circuit_destroy": (None, [_vp]),
+    "bpg_circuit_create_batch": (_i32, [_vp, _sz, C.POINTER(_sz), C.POINTER(_sz), C.POINTER(_sz), C.POINTER(_u32p), C.POINTER(_u32p), C.POINTER(C.c_char_p),
+                                        C.POINTER(_vp)]),
     "bpg_witness_eval": (_i32, [_vp, _sz, _sz, _u32p, _u32p, _u8p, _u8p, _u8p, _u8p, _u8p]),
+    "bpg_witness_eval_batch": (_i32, [_vp, _sz, C.POINTER(_sz), C.POINTER(_sz), C.POINTER(_u32p), C.POINTER(_u32p), C.POINTER(C.c_char_p),
+                                      C.POINTER(C.c_char_p), C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp)]),
     "bpg_r1cs_prove": (C.c_long, [_vp, _vp, _u8p, _sz, _u8p, _u8p, _u8p, _u8p, _u8p, _u8p, C.c_uint, _u8p, _u8p, _sz]),
     "bpg_r1cs_prove_prefetch": (_i32, [_vp, _vp, _u8p, _sz, _u8p, _u8p, _u8p, C.c_uint]),
     "bpg_r1cs_prove_batch": (_i32, [_vp, _sz, C.POINTER(_vp), C.POINTER(C.c_char_p), C.POINTER(_sz), C.POINTER(C.c_char_p), C.POINTER(C.c_char_p),

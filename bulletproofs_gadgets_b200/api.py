@@ -8,6 +8,7 @@ Names follow the bulletproofs fork as the reference calls it (SURVEY.md section 
   mimc_hash(bytes)                                src/mimc_hash/mimc.rs:61
 Scalars are Python ints or 32-byte LE bytes; points are 32-byte compressed ristretto255.
 """
+import array
 import ctypes as C
 import json
 import os
@@ -27,6 +28,12 @@ def _sb(x):
         assert len(x) == 32
         return bytes(x)
     return int(x % L_ORDER).to_bytes(32, "little")
+
+
+def _u32_array(xs):
+    """ctypes uint32 array holding xs (at least one element, so that an empty list still gives a valid pointer)"""
+    a = array.array("I", xs or [0])
+    return (C.c_uint32 * len(a)).from_buffer(a)
 
 
 class Context:
@@ -157,6 +164,39 @@ class Context:
         self.check(self.lib.bpg_mimc_sponge_batch(self.h, flat, (C.c_uint32 * (n + 1))(*offs), n, out, tr))
         raw = out.raw  # (.raw copies the whole buffer: take it once)
         return [raw[32 * i:32 * i + 32] for i in range(n)], (tr.raw if trace else None)
+
+    # ---- batched set-up
+    def circuit_create_batch(self, csrs):
+        """csrs: list of (n, m, row_ptr, term_var, term_coeff bytes) -> list of circuit handles (c_void_p), handle i behaving as
+        the one bpg_circuit_create makes for csrs[i].  All handles share one device allocation; release each with
+        bpg_circuit_destroy, in any order."""
+        k = len(csrs)
+        if k == 0:
+            return []
+        rps, tvs = [_u32_array(c[2]) for c in csrs], [_u32_array(c[3]) for c in csrs]
+        u32pp = lambda xs: (C.POINTER(C.c_uint32) * k)(*[C.cast(x, C.POINTER(C.c_uint32)) for x in xs])
+        sizes = lambda j: (C.c_size_t * k)(*[c[j] for c in csrs])
+        out = (C.c_void_p * k)()
+        self.check(self.lib.bpg_circuit_create_batch(self.h, k, sizes(0), sizes(1), (C.c_size_t * k)(*[len(c[2]) - 1 for c in csrs]), u32pp(rps), u32pp(tvs),
+                                                     (C.c_char_p * k)(*[bytes(c[4]) for c in csrs]), out))
+        return [C.c_void_p(h) for h in out]
+
+    def witness_eval_batch(self, items):
+        """items: list of (n, m, lc_ptr, term_var, term_coeff bytes, v bytes, a_L inputs, a_R inputs (n x 32 bytes or shorter,
+        zero-padded)) -> list of (a_L, a_R, a_O) bytes, entry i being what bpg_witness_eval computes for items[i]"""
+        k = len(items)
+        if k == 0:
+            return []
+        bufs = [[C.create_string_buffer(bytes(it[6]), 32 * max(1, it[0])), C.create_string_buffer(bytes(it[7]), 32 * max(1, it[0])),
+                 C.create_string_buffer(32 * max(1, it[0]))] for it in items]
+        ptrs, tvs = [_u32_array(it[2]) for it in items], [_u32_array(it[3]) for it in items]
+        u32pp = lambda xs: (C.POINTER(C.c_uint32) * k)(*[C.cast(x, C.POINTER(C.c_uint32)) for x in xs])
+        sizes = lambda j: (C.c_size_t * k)(*[it[j] for it in items])
+        bytes_pp = lambda j: (C.c_char_p * k)(*[bytes(it[j]) for it in items])
+        out_pp = lambda j: (C.c_void_p * k)(*[C.addressof(b[j]) for b in bufs])
+        self.check(self.lib.bpg_witness_eval_batch(self.h, k, sizes(0), sizes(1), u32pp(ptrs), u32pp(tvs), bytes_pp(4), bytes_pp(5),
+                                                   out_pp(0), out_pp(1), out_pp(2)))
+        return [tuple(b[j].raw[:32 * it[0]] for j in range(3)) for b, it in zip(bufs, items)]
 
     # ---- batched proving
     def prove_batch(self, items, flags=0):
@@ -370,10 +410,18 @@ class _ConstraintSystem:
             self._w_coeff += int(c % L_ORDER).to_bytes(32, "little")
         self._w_ptr.append(len(self._w_var))
 
+    def _witness_cached(self):
+        return self._witness is not None and self._witness[0] == (self.num_vars, len(self.v))
+
+    def _witness_args(self):
+        """the arguments of bpg_witness_eval as one item of Context.witness_eval_batch"""
+        enc = lambda xs: b"".join(int(x).to_bytes(32, "little") for x in xs)
+        return (self.num_vars, len(self.v), self._w_ptr, self._w_var, bytes(self._w_coeff), enc(self.v), enc(self._in_L), enc(self._in_R))
+
     def witness_bytes(self):
         """(a_L, a_R, a_O) as n x 32-byte LE strings, computed by bpg_witness_eval (cached until the system grows)"""
         n, m = self.num_vars, len(self.v)
-        if self._witness is not None and self._witness[0] == (n, m):
+        if self._witness_cached():
             return self._witness[1]
         enc = lambda xs: b"".join(int(x).to_bytes(32, "little") for x in xs)
         aL, aR = C.create_string_buffer(enc(self._in_L), 32 * max(1, n)), C.create_string_buffer(enc(self._in_R), 32 * max(1, n))
@@ -442,6 +490,10 @@ class _ConstraintSystem:
         return self.num_vars
 
     get_num_vars = get_num_multiplications
+
+    def _circuit_args(self, m):
+        """the arguments of bpg_circuit_create as one entry of Context.circuit_create_batch"""
+        return self.num_vars, m, self.row_ptr, self.term_var, bytes(self.term_coeff)
 
     def _circuit(self, m):
         lib, h = self.ctx.lib, C.c_void_p()
@@ -515,13 +567,13 @@ def prove_batch(provers, bp_gens, ext_rngs=None, flags=0):
     if len(exts) != len(provers):
         raise ValueError("prove_batch: %d ext_rngs for %d provers" % (len(exts), len(provers)))
     enc = lambda xs: b"".join(int(x).to_bytes(32, "little") for x in xs)
-    circs = []
+    # set-up in two calls: every witness not yet cached (bpg_witness_eval_batch), every circuit (bpg_circuit_create_batch)
+    stale = list({id(p): p for p in provers if not p._witness_cached()}.values())
+    for p, w in zip(stale, ctx.witness_eval_batch([p._witness_args() for p in stale])):
+        p._witness = ((p.num_vars, len(p.v)), w)
+    circs = ctx.circuit_create_batch([p._circuit_args(len(p.v)) for p in provers])
     try:
-        items = []
-        for p, ext in zip(provers, exts):
-            circs.append(p._circuit(len(p.v)))
-            aL, aR, aO = p.witness_bytes()
-            items.append((circs[-1], p.label, aL, aR, aO, enc(p.v), enc(p.v_blinding), ext))
+        items = [(c, p.label, *p.witness_bytes(), enc(p.v), enc(p.v_blinding), ext) for c, p, ext in zip(circs, provers, exts)]
         out = ctx.prove_batch(items, flags)
     finally:
         for c in circs:
@@ -559,6 +611,28 @@ class Verifier(_ConstraintSystem):
             self.ctx.lib.bpg_circuit_destroy(circ)
         if not acc.value:
             raise R1CSError("VerificationError")
+
+
+def verify_batch(verifiers, proofs, ext_rngs=None, flags=0):
+    """Verifier::verify of many statements in ONE call (bpg_r1cs_verify_batch) -> list of bool, entry i being whether
+    verifiers[i].verify(proofs[i], ext_rng32=ext_rngs[i], flags=flags) succeeds.  The verifiers share one context; their
+    circuits are made by one bpg_circuit_create_batch.  ext_rngs (one 32-byte string per verifier) default to os.urandom."""
+    if len(proofs) != len(verifiers):
+        raise ValueError("verify_batch: %d proofs for %d verifiers" % (len(proofs), len(verifiers)))
+    if not verifiers:
+        return []
+    ctx = verifiers[0].ctx
+    if any(v.ctx is not ctx for v in verifiers):
+        raise ValueError("verify_batch: every verifier must use the same Context")
+    exts = list(ext_rngs) if ext_rngs is not None else [os.urandom(32) for _ in verifiers]
+    if len(exts) != len(verifiers):
+        raise ValueError("verify_batch: %d ext_rngs for %d verifiers" % (len(exts), len(verifiers)))
+    circs = ctx.circuit_create_batch([v._circuit_args(len(v.V)) for v in verifiers])
+    try:
+        return ctx.verify_batch([(c, v.label, b"".join(v.V), bytes(pf), ext) for c, v, pf, ext in zip(circs, verifiers, proofs, exts)], flags)
+    finally:
+        for c in circs:
+            ctx.lib.bpg_circuit_destroy(c)
 
 
 def mimc_hash(preimage, ctx=None):

@@ -93,10 +93,11 @@ __device__ __forceinline__ void block_sum_rows(sc *acc, const sc *__restrict__ r
     block_sum_scalars<NS>(acc, smem);
 }
 
+__device__ __forceinline__ void sc_reduce_at(sc *v, uint32_t i) { sc x; ld_sc(x, &v[i]); sc_reduce(x, x); st_sc(&v[i], x); }
 __global__ void __launch_bounds__(256) k_sc_reduce_inplace(sc *v, uint32_t n) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    sc x; ld_sc(x, &v[i]); sc_reduce(x, x); st_sc(&v[i], x);
+    sc_reduce_at(v, i);
 }
 // Scalar::from_bytes_mod_order_wide of one raw 64-byte TranscriptRng draw
 __device__ __forceinline__ void reduce_wide_draw(sc &r, const uint32_t *__restrict__ raw) {
@@ -409,46 +410,77 @@ __device__ __forceinline__ void lc_eval(sc &acc, uint32_t t0, uint32_t t1, const
         sc_add_r(acc, acc, p);
     }
 }
-__global__ void __launch_bounds__(128) k_witness_level(const uint32_t *__restrict__ order, uint32_t k0, uint32_t k1, const uint32_t *__restrict__ lc_ptr,
-                                                        const uint32_t *__restrict__ term_var, const sc *__restrict__ term_coeff, sc *aL, sc *aR, sc *aO,
-                                                        const sc *__restrict__ v) {
-    uint32_t k = k0 + blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= k1) return;
-    uint32_t i = order[k];
+// Multiplier i made by multiply(left_i, right_i): a_L[i] = <left_i>, a_R[i] = <right_i>, a_O[i] = a_L[i] a_R[i]
+__device__ __forceinline__ void witness_multiply(uint32_t i, const uint32_t *__restrict__ lc_ptr, const uint32_t *__restrict__ term_var,
+                                                 const sc *__restrict__ term_coeff, sc *aL, sc *aR, sc *aO, const sc *__restrict__ v) {
     sc l, r, o;
     lc_eval(l, lc_ptr[2 * i], lc_ptr[2 * i + 1], term_var, term_coeff, aL, aR, aO, v);
     lc_eval(r, lc_ptr[2 * i + 1], lc_ptr[2 * i + 2], term_var, term_coeff, aL, aR, aO, v);
     sc_mul(o, l, r);
     st_sc(&aL[i], l); st_sc(&aR[i], r); st_sc(&aO[i], o);
 }
+// Multiplier i assigned directly by the caller (allocate_multiplier / allocate): a_O[i] = a_L[i] a_R[i]
+__device__ __forceinline__ void witness_assigned(uint32_t i, const sc *aL, const sc *aR, sc *aO) {
+    sc l, r, o;
+    ld_sc(l, &aL[i]); ld_sc(r, &aR[i]);
+    sc_mul(o, l, r);
+    st_sc(&aO[i], o);
+}
+__global__ void __launch_bounds__(128) k_witness_level(const uint32_t *__restrict__ order, uint32_t k0, uint32_t k1, const uint32_t *__restrict__ lc_ptr,
+                                                        const uint32_t *__restrict__ term_var, const sc *__restrict__ term_coeff, sc *aL, sc *aR, sc *aO,
+                                                        const sc *__restrict__ v) {
+    uint32_t k = k0 + blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= k1) return;
+    witness_multiply(order[k], lc_ptr, term_var, term_coeff, aL, aR, aO, v);
+}
 // A run of consecutive NARROW levels (a MiMC chain is 972 levels of one multiplier each) in ONE launch: a single block walks the
 // levels [l0, l1) with a barrier between them instead of one launch per level (~0.7 us against ~3 us per level).
+__device__ __forceinline__ void witness_walk_levels(const uint32_t *__restrict__ order, const uint32_t *__restrict__ lptr, uint32_t l0, uint32_t l1,
+                                                    const uint32_t *__restrict__ lc_ptr, const uint32_t *__restrict__ term_var,
+                                                    const sc *__restrict__ term_coeff, sc *aL, sc *aR, sc *aO, const sc *__restrict__ v) {
+    for (uint32_t l = l0; l < l1; l++) {
+        const uint32_t k1 = lptr[l + 1];
+        for (uint32_t k = lptr[l] + threadIdx.x; k < k1; k += blockDim.x) witness_multiply(order[k], lc_ptr, term_var, term_coeff, aL, aR, aO, v);
+        __syncthreads(); // the next level reads what this one wrote (same block: the barrier orders the global accesses)
+    }
+}
 __global__ void __launch_bounds__(256) k_witness_levels_block(const uint32_t *__restrict__ order, const uint32_t *__restrict__ lptr, uint32_t l0, uint32_t l1,
                                                                const uint32_t *__restrict__ lc_ptr, const uint32_t *__restrict__ term_var,
                                                                const sc *__restrict__ term_coeff, sc *aL, sc *aR, sc *aO, const sc *__restrict__ v) {
-    for (uint32_t l = l0; l < l1; l++) {
-        const uint32_t k1 = lptr[l + 1];
-        for (uint32_t k = lptr[l] + threadIdx.x; k < k1; k += blockDim.x) {
-            uint32_t i = order[k];
-            sc a, b, o;
-            lc_eval(a, lc_ptr[2 * i], lc_ptr[2 * i + 1], term_var, term_coeff, aL, aR, aO, v);
-            lc_eval(b, lc_ptr[2 * i + 1], lc_ptr[2 * i + 2], term_var, term_coeff, aL, aR, aO, v);
-            sc_mul(o, a, b);
-            st_sc(&aL[i], a); st_sc(&aR[i], b); st_sc(&aO[i], o);
-        }
-        __syncthreads(); // the next level reads what this one wrote (same block: the barrier orders the global accesses)
-    }
+    witness_walk_levels(order, lptr, l0, l1, lc_ptr, term_var, term_coeff, aL, aR, aO, v);
 }
 // a_O = a_L a_R for the multipliers the caller assigned directly (allocate_multiplier / allocate)
 __global__ void __launch_bounds__(128) k_witness_assigned(const uint32_t *__restrict__ order, uint32_t k1, const sc *__restrict__ aL, const sc *__restrict__ aR,
                                                            sc *__restrict__ aO) {
     uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= k1) return;
-    uint32_t i = order[k];
-    sc l, r, o;
-    ld_sc(l, &aL[i]); ld_sc(r, &aR[i]);
-    sc_mul(o, l, r);
-    st_sc(&aO[i], o);
+    witness_assigned(order[k], aL, aR, aO);
+}
+
+// bpg_witness_eval_batch: the statements of a pass at ragged offsets of shared regions, one block per statement.  Term indices
+// and multiplier indices stay those of the statement: the block offsets the base pointers instead.
+struct wb_desc {
+    uint32_t n, m, T, depth;
+    uint32_t noff;  // multipliers: a_L, a_R, a_O and order at noff
+    uint32_t moff;  // committed values
+    uint32_t toff;  // terms (coefficients and variables)
+    uint32_t poff;  // lc_ptr (2n + 1 entries)
+    uint32_t loff;  // level pointers (depth + 2 entries)
+};
+__global__ void __launch_bounds__(256) k_witness_batch(const wb_desc *__restrict__ D, const uint32_t *__restrict__ order, const uint32_t *__restrict__ lptr,
+                                                        const uint32_t *__restrict__ lc_ptr, const uint32_t *__restrict__ term_var, sc *term_coeff,
+                                                        sc *aL, sc *aR, sc *aO, sc *v) {
+    const wb_desc d = D[blockIdx.x];
+    aL += d.noff; aR += d.noff; aO += d.noff; v += d.moff; term_coeff += d.toff;
+    order += d.noff; lptr += d.loff; lc_ptr += d.poff; term_var += d.toff;
+    // the caller's inputs, reduced in place as k_sc_reduce_inplace does (Scalar::from_bits semantics)
+    for (uint32_t k = threadIdx.x; k < d.T; k += blockDim.x) sc_reduce_at(term_coeff, k);
+    for (uint32_t k = threadIdx.x; k < d.n; k += blockDim.x) { sc_reduce_at(aL, k); sc_reduce_at(aR, k); }
+    for (uint32_t k = threadIdx.x; k < d.m; k += blockDim.x) sc_reduce_at(v, k);
+    __syncthreads();
+    for (uint32_t k = threadIdx.x; k < lptr[1]; k += blockDim.x) witness_assigned(order[k], aL, aR, aO);
+    __syncthreads();
+    witness_walk_levels(order, lptr, 1, d.depth + 1, lc_ptr, term_var, term_coeff, aL, aR, aO, v);
 }
 
 // ---------------------------------------------------------------- BPG_FLAG_FAST_BLINDING: s_L, s_R on the device

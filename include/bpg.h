@@ -141,6 +141,19 @@ int bpg_mimc_sponge_batch(bpg_ctx *ctx, const uint8_t *blocks, const uint32_t *b
 int bpg_circuit_create(bpg_ctx *ctx, size_t n_multipliers, size_t m_commitments, size_t q_constraints,
                        const uint32_t *row_ptr, const uint32_t *term_var, const uint8_t *term_coeff, bpg_circuit **out);
 void bpg_circuit_destroy(bpg_circuit *c);
+/* K circuits in one call.  Handle out[i] behaves exactly as the one bpg_circuit_create(ctx, n_multipliers[i], m_commitments[i],
+ * q_constraints[i], row_ptr[i], term_var[i], term_coeff[i], ...) makes, in bpg_r1cs_prove, _prefetch, _prove_batch,
+ * bpg_r1cs_verify and _verify_batch.
+ *  - Every argument of every circuit is checked before any device work: a NULL array or entry where bpg_circuit_create needs
+ *    a pointer, a term whose index is out of range or whose kind is not 0..4, or n, m >= 2^22 fail the whole call with the
+ *    code bpg_circuit_create returns for the first such circuit (BPG_E_ARG / BPG_E_SIZE); every out[i] is NULL then.
+ *    count = 0 returns BPG_OK.
+ *  - All circuits of the call share one device allocation, filled by one copy (bpg_circuit_create is the count-1 case: one
+ *    cudaMalloc per circuit).  Each handle is released by bpg_circuit_destroy, in any order; the allocation is freed with the
+ *    last handle of the call. */
+int bpg_circuit_create_batch(bpg_ctx *ctx, size_t count, const size_t *n_multipliers, const size_t *m_commitments,
+                             const size_t *q_constraints, const uint32_t *const *row_ptr, const uint32_t *const *term_var,
+                             const uint8_t *const *term_coeff, bpg_circuit **out);
 
 /* Witness evaluation on the device (SURVEY 8 f-3).  Multiplier i created by ConstraintSystem::multiply(left_i, right_i) has
  * a_L[i] = <left_i>, a_R[i] = <right_i>, a_O[i] = a_L[i] a_R[i], the linear combinations being evaluated over the assignment so
@@ -152,6 +165,21 @@ void bpg_circuit_destroy(bpg_circuit *c);
  * single-block launch. */
 int bpg_witness_eval(bpg_ctx *ctx, size_t n, size_t m, const uint32_t *lc_ptr, const uint32_t *term_var, const uint8_t *term_coeff,
                      const uint8_t *v, uint8_t *aL, uint8_t *aR, uint8_t *aO);
+/* K witnesses in one call.  Entry i leaves aL[i], aR[i], aO[i] byte-identical to
+ * bpg_witness_eval(ctx, n[i], m[i], lc_ptr[i], term_var[i], term_coeff[i], v[i], aL[i], aR[i], aO[i]).
+ * The statements with n <= 4096 are evaluated together: one upload, one launch (one block per statement, its levels walked
+ * with a barrier between them), one read-back per pass; a statement with a larger n is evaluated as bpg_witness_eval does
+ * inside the call, so any mix may be passed.
+ *  - Every argument of every statement is checked before any device work: a NULL array or entry where bpg_witness_eval needs
+ *    a pointer, lc_ptr ranges that are not nested in [0, T], a term referencing a later multiplier or a commitment out of
+ *    range, a bad kind, or n, m >= 2^22 fail the whole call with the code bpg_witness_eval returns (BPG_E_ARG / BPG_E_SIZE)
+ *    for the first such statement; no caller buffer is written then (aL, aR included).  count = 0 returns BPG_OK.
+ *  - The witness is wiped from the device scratch and the host staging buffer before the call returns.
+ *  - count has no upper limit: the batch is split internally into passes of at most 1024 statements, 2^17 multipliers and
+ *    2^20 terms plus committed values (a statement above that is a pass of its own), with unchanged bytes. */
+int bpg_witness_eval_batch(bpg_ctx *ctx, size_t count, const size_t *n, const size_t *m, const uint32_t *const *lc_ptr,
+                           const uint32_t *const *term_var, const uint8_t *const *term_coeff, const uint8_t *const *v,
+                           uint8_t *const *aL, uint8_t *const *aR, uint8_t *const *aO);
 
 /* Prover::new(label) + commit(v_i, blinding_i)* + (constraints) + prove(&bp_gens)  [ext; prover.rs:52-54,93
  * gadget.rs:18-38].  Writes the m commitments to V_out (nullable) and the serialised R1CSProof to `proof`;

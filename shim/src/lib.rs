@@ -157,18 +157,22 @@ impl Device {
         let k = jobs.len();
         let mut ext = vec![0u8; 32 * k];
         rand::thread_rng().fill_bytes(&mut ext);
-        let mut circuits: Vec<*mut ffi::BpgCircuit> = Vec::with_capacity(k);
         for j in jobs {
-            let (n, m) = (j.a_l.len() / 32, j.v.len() / 32);
             assert!(j.a_r.len() == j.a_l.len() && j.a_o.len() == j.a_l.len() && j.v_blinding.len() == j.v.len());
-            let mut circuit = ptr::null_mut();
-            let rc = unsafe { ffi::bpg_circuit_create(self.ctx, n, m, j.cs.rows(), j.cs.row_ptr.as_ptr(), j.cs.term_var.as_ptr(), j.cs.term_coeff.as_ptr(), &mut circuit) };
-            if rc != ffi::BPG_OK {
-                for c in &circuits { unsafe { ffi::bpg_circuit_destroy(*c) } }
-                return Err(Device::error(self.ctx, rc));
-            }
-            circuits.push(circuit);
         }
+        // every circuit in one call (one device allocation shared by the k handles)
+        let ns: Vec<usize> = jobs.iter().map(|j| j.a_l.len() / 32).collect();
+        let ms: Vec<usize> = jobs.iter().map(|j| j.v.len() / 32).collect();
+        let qs: Vec<usize> = jobs.iter().map(|j| j.cs.rows()).collect();
+        let row_ptrs: Vec<*const u32> = jobs.iter().map(|j| j.cs.row_ptr.as_ptr()).collect();
+        let term_vars: Vec<*const u32> = jobs.iter().map(|j| j.cs.term_var.as_ptr()).collect();
+        let term_coeffs: Vec<*const u8> = jobs.iter().map(|j| j.cs.term_coeff.as_ptr()).collect();
+        let mut circuits: Vec<*mut ffi::BpgCircuit> = vec![ptr::null_mut(); k];
+        let rc = unsafe {
+            ffi::bpg_circuit_create_batch(self.ctx, k, ns.as_ptr(), ms.as_ptr(), qs.as_ptr(), row_ptrs.as_ptr(), term_vars.as_ptr(), term_coeffs.as_ptr(),
+                                          circuits.as_mut_ptr())
+        };
+        self.check(rc)?;
         let cap = 1 + 32 * (14 + 64 + 2);
         let mut proofs: Vec<Vec<u8>> = (0..k).map(|_| vec![0u8; cap]).collect();
         let mut vouts: Vec<Vec<u8>> = jobs.iter().map(|j| vec![0u8; std::cmp::max(j.v.len(), 32)]).collect();

@@ -25,8 +25,8 @@ def param(p):
         return name, "*const *mut BpgCircuit"
     if stars == 2 and const and base == "uint8_t" and not ty.startswith("const"):  # uint8_t *const *proofs
         return name, "*const *mut u8"
-    if stars == 2 and const and base == "uint8_t":       # const uint8_t *const *labels
-        return name, "*const *const u8"
+    if stars == 2 and const and base in ("uint8_t", "uint32_t"):  # const uint8_t *const *labels, const uint32_t *const *row_ptr
+        return name, "*const *const " + BASE[base]
     rt = BASE[base]
     for i in range(stars):
         rt = ("*const " if const else "*mut ") + rt
