@@ -995,3 +995,4 @@ extern "C" int bpg_host_rng_draw64(const uint8_t *label, size_t label_len, const
 #include "prover.inl"
 #include "prover_batch.inl"
 #include "witness_batch.inl"
+#include "verify_batch.inl"

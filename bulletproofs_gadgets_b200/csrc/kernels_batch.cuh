@@ -1,5 +1,5 @@
-// kernels_batch.cuh -- ragged (many-proof) versions of the prover's vector kernels and a many-output small MSM, for
-// bpg_r1cs_prove_batch (prover_batch.inl).
+// kernels_batch.cuh -- ragged (many-proof) versions of the prover's and the verifier's vector kernels and a many-output
+// small MSM, for bpg_r1cs_prove_batch (prover_batch.inl) and bpg_r1cs_verify_batch (verify_batch.inl).
 //
 // The K proofs of a batch keep their vectors at ragged offsets off_p = sum_{k<p} N_k of shared buffers.  A kernel either
 // walks 128-element blocks of those vectors -- blkp[block] = proof, the element index is (block - blk0_p) * 128 + thread --
@@ -23,6 +23,7 @@ struct pb_desc {
     uint32_t vc0, sp0; // prefix counts of virtual columns / split columns of the earlier proofs
     uint32_t nv, nsplit;
     uint32_t pt, nz, ny; // power tables of this proof: z at pt, y at pt + nz, y^-1 at pt + nz + ny (PB_POW_LO + hi entries each)
+    uint32_t st, slot;   // bpg_r1cs_verify_batch only: s table (ny entries) at st of the table array, delta | wV | wc at slot
     const uint32_t *vcol_ptr, *vcol_dst, *row, *split;
     const sc *coeff;
 };
@@ -207,6 +208,78 @@ __global__ void __launch_bounds__(128) k_pb_final_ab(const pb_desc *__restrict__
     sc x;
     ld_sc(x, &a[D[p].off]); st_sc(&out[2 * p], x);
     ld_sc(x, &b[D[p].off]); st_sc(&out[2 * p + 1], x);
+}
+
+// ---- bpg_r1cs_verify_batch (verify_batch.inl): the verifier's scalar preparation of the K proofs of a pass.  The descriptors
+// are pb_desc with off = g | h of the proof (g at off, h at off + N, relative to the pass's gh base) and the small scalars use
+// the prover's stride with the verifier's meaning:
+//   small[PB_SLOTS p + k]:  [0] x  [1] a  [2] b  [3] y  [4] z  [5] y^-1  [6] u  [7] allinv      usq[VB_LGMAX p + j] = u_j^2
+// (k_pb_pow_tables also builds the y table there, which the verifier does not read.)
+#define VB_LGMAX 12u // lg N of BPG_BATCH_MAX_N
+// s tables of every proof, one thread per entry; the proofs' tables are at D[p].st (non-decreasing), st0 .. st0 + total
+__global__ void __launch_bounds__(128) k_pb_s_tables(const pb_desc *__restrict__ D, uint32_t K, uint32_t st0, uint32_t total, const sc *__restrict__ small,
+                                                     const sc *__restrict__ usq, sc *__restrict__ pt) {
+    uint32_t g = blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= total) return;
+    g += st0;
+    const uint32_t p = pb_find(D, K, g, [](const pb_desc &d) { return d.st; });
+    sc acc;
+    s_table_entry<PB_POW_LG>(acc, g - D[p].st, usq + VB_LGMAX * p, &small[PB_SLOTS * p + 7], D[p].lgN);
+    st_sc(&pt[g], acc);
+}
+// k_verify_scalars, one 128-element block of one proof per block: g | h of the proof, dparts[block] = the block's share of delta
+__global__ void __launch_bounds__(128) k_pb_verify_scalars(const pb_desc *__restrict__ D, const uint32_t *__restrict__ blkp, const sc *__restrict__ small,
+                                                           const sc *__restrict__ w, const sc *__restrict__ pt, sc *__restrict__ gh, sc *__restrict__ dparts) {
+    __shared__ sc smem[128];
+    const uint32_t p = blkp[blockIdx.x];
+    const pb_desc &P = D[p];
+    const uint32_t i = (blockIdx.x - P.blk0) * 128u + threadIdx.x;
+    sc d;
+    sc_zero(d);
+    if (i < P.N) {
+        const sc *sm = small + PB_SLOTS * p, *yit = pt + P.pt + P.nz + P.ny, *stab = pt + P.st;
+        sc x, ia, ib, u;
+        ld_sc(x, &sm[0]); ld_sc(ia, &sm[1]); ld_sc(ib, &sm[2]); ld_sc(u, &sm[6]);
+        sc *g = gh + P.off;
+        verify_scalars_elem<PB_POW_LG>(i, P.n, P.N, x, ia, ib, u, w + P.woff, yit, yit + PB_POW_LO, stab, stab + PB_POW_LO, g, g + P.N, d);
+    }
+    block_sum_scalars<1>(&d, smem);
+    if (threadIdx.x == 0) st_sc(&dparts[blockIdx.x], d);
+}
+// one block per proof: delta (sum of the proof's block partials), wV[0..m), wc -> slots[slot_p ..] (m + 2 scalars per proof)
+__global__ void __launch_bounds__(128) k_pb_verify_out(const pb_desc *__restrict__ D, const sc *__restrict__ dparts, const sc *__restrict__ w,
+                                                       sc *__restrict__ slots) {
+    __shared__ sc smem[128];
+    const pb_desc &P = D[blockIdx.x];
+    sc acc;
+    block_sum_rows<1>(&acc, dparts, P.blk0, (P.N + 127u) / 128u, smem);
+    sc *o = slots + P.slot;
+    if (threadIdx.x == 0) st_sc(&o[0], acc);
+    for (uint32_t k = threadIdx.x; k <= P.m; k += 128) { sc x; ld_sc(x, &w[P.woff + 3 * P.n + k]); st_sc(&o[1 + k], x); }
+}
+// Combined check of a set of proofs (verify_finish): acc[i] = sum_t rho_t g_t[i], acc[Nmax + i] = sum_t rho_t h_t[i] over the
+// terms with i < N_t (h_t = g_t + N_t).  The terms are sorted by N_t, largest first.  One thread per output scalar.
+struct vb_term {
+    sc rho;
+    const sc *g;
+    uint32_t N, pad;
+};
+__global__ void __launch_bounds__(128) k_pb_axpy_gh(const vb_term *__restrict__ T, uint32_t nt, uint32_t Nmax, sc *__restrict__ acc) {
+    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= 2 * Nmax) return;
+    const uint32_t side = t >= Nmax ? 1u : 0u, i = t - side * Nmax;
+    sc a;
+    sc_zero(a);
+#pragma unroll 1
+    for (uint32_t k = 0; k < nt; k++) {
+        const uint32_t N = T[k].N;
+        if (i >= N) break;
+        sc x, r, p;
+        ld_sc(x, &T[k].g[side * N + i]); ld_sc(r, &T[k].rho);
+        sc_mul(p, r, x);
+        sc_add_r(a, a, p);
+    }
+    st_sc(&acc[t], a);
 }
 
 // ---- many-output small MSM (msm_run_many): k_msm_digits<*, SPLIT = 1> with the segments in a device table (any number of

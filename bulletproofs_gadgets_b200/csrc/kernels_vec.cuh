@@ -336,15 +336,13 @@ __global__ void __launch_bounds__(128) k_ipp_fold(uint32_t N, uint32_t nj, const
 }
 
 // ---------------------------------------------------------------- verifier scalars (a8)
-// stab_lo[t] = allinv * prod_{bit k of t set} usq[lg-1-k]  (t < 1024, bits k < min(lg,10))
-// stab_hi[j] = prod_{bit k of j set} usq[lg-1-(k+10)]
-__global__ void __launch_bounds__(128) k_s_tables(const sc *__restrict__ usq, const sc *__restrict__ allinv, uint32_t lg, sc *__restrict__ lo,
-                                                   sc *__restrict__ hi, uint32_t nhi) {
-    uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= 1024 + nhi) return;
-    sc acc;
+// Entry t of the s tables, split like a power table with a 2^LO-entry low part (bpg_r1cs_verify: LO = 10, the batch
+// verifier: LO = 6):  lo[t] = allinv * prod_{bit k of t set} usq[lg-1-k]  (t < 2^LO, bits k < min(lg, LO))
+//                     hi[j] = prod_{bit k of j set} usq[lg-1-(k+LO)]      (t = 2^LO + j)
+template <int LO>
+__device__ __forceinline__ void s_table_entry(sc &acc, uint32_t t, const sc *__restrict__ usq, const sc *__restrict__ allinv, uint32_t lg) {
     uint32_t idx, shift;
-    if (t < 1024) { ld_sc(acc, allinv); idx = t; shift = 0; } else { sc_set_u32(acc, 1); idx = t - 1024; shift = 10; }
+    if (t < (1u << LO)) { ld_sc(acc, allinv); idx = t; shift = 0; } else { sc_set_u32(acc, 1); idx = t - (1u << LO); shift = LO; }
 #pragma unroll 1
     for (uint32_t k = 0; k < 22; k++) {
         if (!((idx >> k) & 1u)) continue;
@@ -353,40 +351,52 @@ __global__ void __launch_bounds__(128) k_s_tables(const sc *__restrict__ usq, co
         sc f; ld_sc(f, &usq[lg - 1 - bit]);
         sc_mul(acc, acc, f);
     }
+}
+__global__ void __launch_bounds__(128) k_s_tables(const sc *__restrict__ usq, const sc *__restrict__ allinv, uint32_t lg, sc *__restrict__ lo,
+                                                   sc *__restrict__ hi, uint32_t nhi) {
+    uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= 1024 + nhi) return;
+    sc acc;
+    s_table_entry<10>(acc, t, usq, allinv, lg);
     if (t < 1024) st_sc(&lo[t], acc); else st_sc(&hi[t - 1024], acc);
 }
-// g_i = uf (x y^-i wR_i - a s_i) ; h_i = uf (y^-i (x wL_i + wO_i - b s_{N-1-i}) - 1) ; delta partials <y^-i wR_i, wL_i>
-// vs = [x, a, b, u]
+// g_i = uf (x y^-i wR_i - a s_i) ; h_i = uf (y^-i (x wL_i + wO_i - b s_{N-1-i}) - 1) ; d += <y^-i wR_i, wL_i>   (i < N)
+template <int LO>
+__device__ __forceinline__ void verify_scalars_elem(uint32_t i, uint32_t n, uint32_t N, const sc &x, const sc &ia, const sc &ib, const sc &u,
+                                                    const sc *__restrict__ w, const sc *__restrict__ yilo, const sc *__restrict__ yihi,
+                                                    const sc *__restrict__ slo, const sc *__restrict__ shi, sc *__restrict__ g, sc *__restrict__ hh, sc &d) {
+    sc yinv, s_i, s_r, p, q, gv, hv, one;
+    sc_set_u32(one, 1);
+    pow_lookup<LO>(yinv, yilo, yihi, i);
+    pow_lookup<LO>(s_i, slo, shi, i);
+    pow_lookup<LO>(s_r, slo, shi, N - 1 - i);
+    sc_mul(p, ia, s_i);
+    sc_mul(q, ib, s_r);
+    if (i < n) {
+        sc wl, wr, wo, ywr, t;
+        ld_sc(wl, &w[i]); ld_sc(wr, &w[n + i]); ld_sc(wo, &w[2 * (size_t)n + i]);
+        sc_mul(ywr, yinv, wr);
+        sc_mul(t, ywr, wl); sc_add_r(d, d, t);
+        sc_mul(t, x, ywr); sc_sub_r(gv, t, p);
+        sc_mul(t, x, wl); sc_add_r(t, t, wo); sc_sub_r(t, t, q); sc_mul(hv, yinv, t); sc_sub_r(hv, hv, one);
+    } else {
+        sc z, t; sc_zero(z);
+        sc_sub_r(gv, z, p);
+        sc_sub_r(t, z, q); sc_mul(hv, yinv, t); sc_sub_r(hv, hv, one);
+        sc_mul(gv, gv, u); sc_mul(hv, hv, u);
+    }
+    st_sc(&g[i], gv); st_sc(&hh[i], hv);
+}
+// vs = [x, a, b, u]; dparts[block] = the block's share of delta
 __global__ void __launch_bounds__(128) k_verify_scalars(uint32_t n, uint32_t N, const sc *__restrict__ vs, const sc *__restrict__ w,
                                                          const sc *__restrict__ yilo, const sc *__restrict__ yihi, const sc *__restrict__ slo,
                                                          const sc *__restrict__ shi, sc *__restrict__ g, sc *__restrict__ hh, sc *__restrict__ dparts) {
     __shared__ sc smem[128];
     sc d; sc_zero(d);
-    sc x, ia, ib, u, one;
+    sc x, ia, ib, u;
     ld_sc(x, &vs[0]); ld_sc(ia, &vs[1]); ld_sc(ib, &vs[2]); ld_sc(u, &vs[3]);
-    sc_set_u32(one, 1);
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < N; i += gridDim.x * blockDim.x) {
-        sc yinv, s_i, s_r, p, q, gv, hv;
-        pow_lookup<10>(yinv, yilo, yihi, i);
-        pow_lookup<10>(s_i, slo, shi, i);
-        pow_lookup<10>(s_r, slo, shi, N - 1 - i);
-        sc_mul(p, ia, s_i);
-        sc_mul(q, ib, s_r);
-        if (i < n) {
-            sc wl, wr, wo, ywr, t;
-            ld_sc(wl, &w[i]); ld_sc(wr, &w[n + i]); ld_sc(wo, &w[2 * (size_t)n + i]);
-            sc_mul(ywr, yinv, wr);
-            sc_mul(t, ywr, wl); sc_add_r(d, d, t);
-            sc_mul(t, x, ywr); sc_sub_r(gv, t, p);
-            sc_mul(t, x, wl); sc_add_r(t, t, wo); sc_sub_r(t, t, q); sc_mul(hv, yinv, t); sc_sub_r(hv, hv, one);
-        } else {
-            sc z, t; sc_zero(z);
-            sc_sub_r(gv, z, p);
-            sc_sub_r(t, z, q); sc_mul(hv, yinv, t); sc_sub_r(hv, hv, one);
-            sc_mul(gv, gv, u); sc_mul(hv, hv, u);
-        }
-        st_sc(&g[i], gv); st_sc(&hh[i], hv);
-    }
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < N; i += gridDim.x * blockDim.x)
+        verify_scalars_elem<10>(i, n, N, x, ia, ib, u, w, yilo, yihi, slo, shi, g, hh, d);
     block_sum_scalars<1>(&d, smem);
     if (threadIdx.x == 0) st_sc(&dparts[blockIdx.x], d);
 }
@@ -534,14 +544,4 @@ __global__ void __launch_bounds__(128) k_expand_blinding(const uint64_t *__restr
     sc r;
     sc_reduce512(r, R);
     st_sc(&out[i], r);
-}
-
-// batch verification: Gacc[i] += rho * g[i], Hacc[i] += rho * h[i]  (scalars of proof i folded into the combined check)
-__global__ void __launch_bounds__(128) k_axpy_gh(sc rho, const sc *__restrict__ g, const sc *__restrict__ h, uint32_t n, sc *__restrict__ Gacc,
-                                                  sc *__restrict__ Hacc) {
-    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    sc a, x, p;
-    ld_sc(x, &g[i]); ld_sc(a, &Gacc[i]); sc_mul(p, rho, x); sc_add_r(a, a, p); st_sc(&Gacc[i], a);
-    ld_sc(x, &h[i]); ld_sc(a, &Hacc[i]); sc_mul(p, rho, x); sc_add_r(a, a, p); st_sc(&Hacc[i], a);
 }

@@ -228,7 +228,10 @@ int bpg_r1cs_verify(bpg_ctx *ctx, bpg_circuit *c, const uint8_t *label, size_t l
  * isolated, so verdicts equal one-by-one verification.  ext_rng32 = count x 32 bytes (one thread_rng stand-in per proof):
  * it MUST be fresh secret randomness (the reference draws it from thread_rng inside Verifier::verify).  The combination
  * weights are derived from every proof's label, commitments and full proof bytes together with ext_rng32, so they are
- * bound to the statements being checked and cannot be anticipated by the provers. */
+ * bound to the statements being checked and cannot be anticipated by the provers.  Every transcript is replayed on the
+ * host; the proofs whose replay succeeds and whose padded size N is at most 4096 have their scalars prepared in lockstep,
+ * in passes of at most 1 024 proofs and 2^17 padded elements with a fixed number of launches each, larger proofs one by
+ * one inside the call.  Each combined check of a set of proofs sums their G/H scalars in one launch. */
 int bpg_r1cs_verify_batch(bpg_ctx *ctx, size_t count, bpg_circuit *const *circuits, const uint8_t *const *labels,
                           const size_t *label_lens, const uint8_t *const *V32, const uint8_t *const *proofs,
                           const size_t *proof_lens, const uint8_t *ext_rng32, unsigned flags, int *accept);

@@ -1,91 +1,137 @@
 #!/usr/bin/env python3
-"""BASELINE config 5 shape: many small independent proofs (own transcript each, ~1 % deliberately invalid) verified by
-K concurrent contexts on one GPU; verdicts are checked against the expected ones.  Proof generation (setup) uses the GPU
-prover through the same C ABI."""
-import ctypes as C
+"""Batch verification on the BASELINE configs[4] mix: `total` SET_MEMBER / LESS_THAN statements (statement k false when
+k % 100 == 37, i.e. 1 %), assembled as bench.batch_verify_config5 does and proved on the GPU (bpg_r1cs_prove_batch), then
+verified by `--contexts` contexts in threads, `--per-call` proofs per bpg_r1cs_verify_batch call.  Every per-call size runs
+twice: on the whole mix (1 % invalid, so about half of the 64-proof calls bisect) and on its valid statements only (0 %), so
+the cost of the bisection shows.  Reports verifications/s, launches and host CPU per verification and whether every verdict
+equals the expected one, with a digest of all verdicts (equal digests: equal verdicts, e.g. across library versions).
+Prints one JSON line (and writes it to --out if given).
+
+    python tools/bench_batch_verify.py [--total 8192] [--contexts 8] [--per-call 64,256] [--repeat 3] [--cache path] [--out path]
+
+--cache keeps the assembled statements (front-end output, no proofs) in a pickle, so alternating runs of two library
+versions verify the same statements without assembling them again."""
+import argparse
+import hashlib
 import json
+import multiprocessing as mp
 import os
+import pickle
+import subprocess
 import sys
 import time
 from concurrent.futures import ThreadPoolExecutor
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "tests"))
+
+
+def gpu_info():
+    """(card name, power limit) of device 0 as nvidia-smi reports them, ("unknown", "unknown") if it cannot say"""
+    try:
+        q = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True, text=True)
+    except OSError:
+        return "unknown", "unknown"
+    fields = [x.strip() for x in q.stdout.strip().split(",")]
+    if q.returncode != 0 or len(fields) != 2:
+        return "unknown", "unknown"
+    return fields[0], fields[1]
+
+
+def assemble(total, cache):
+    import bench
+    if cache and os.path.exists(cache):
+        with open(cache, "rb") as f:
+            built = pickle.load(f)
+        if len(built) == total:
+            return built
+    jobs = [("sm" if k % 2 == 0 else "lt", k, (k % 100) != 37) for k in range(total)]
+    with mp.get_context("spawn").Pool(max(1, min(16, os.cpu_count() or 1))) as pool:
+        built = pool.map(bench._cfg5_assemble, jobs, chunksize=32)
+    if cache:
+        with open(cache, "wb") as f:
+            pickle.dump(built, f)
+    return built
 
 
 def main():
     import bulletproofs_gadgets_b200 as bpg
-    import circuits
-    K = int(sys.argv[1]) if len(sys.argv) > 1 else 16
-    total = int(sys.argv[2]) if len(sys.argv) > 2 else 2048
-    ctxs = [bpg.Context(0) for _ in range(K)]
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--total", type=int, default=8192)
+    ap.add_argument("--contexts", type=int, default=8)
+    ap.add_argument("--per-call", default="64,256")
+    ap.add_argument("--repeat", type=int, default=3)
+    ap.add_argument("--cache", default=None)
+    ap.add_argument("--out", default=None)
+    args = ap.parse_args()
+    name, power = gpu_info()
+    built = assemble(args.total, args.cache)
+    NCTX = args.contexts
+    ctxs = [bpg.Context(0) for _ in range(NCTX)]
     for c in ctxs:
         c.gens_ensure(512)
-    shapes = {}
-    items = []
-    for k in range(total):
-        nm = 100 + (k % 5) * 90          # 100 .. 460 multipliers (the set_membership / less_than range of SURVEY 8a config 5)
-        wrong = (k % 101 == 7)
-        inst = circuits.chain_instance(nm, 7000 + (k % 40), wrong=wrong) if (nm, wrong, k % 40) not in shapes else shapes[(nm, wrong, k % 40)]
-        shapes[(nm, wrong, k % 40)] = inst
-        items.append((inst, not wrong))
-    # one circuit handle per (context, shape); proofs made once per shape on context 0
-    proofs = {}
-    handles = [dict() for _ in range(K)]
-    for key, inst in shapes.items():
-        rp, tv, tc = inst["csr"]
-        for ci, c in enumerate(ctxs):
-            h = C.c_void_p()
-            c.check(c.lib.bpg_circuit_create(c.h, inst["n"], 3, len(rp) - 1, (C.c_uint32 * len(rp))(*rp), (C.c_uint32 * max(1, len(tv)))(*tv), tc, C.byref(h)))
-            handles[ci][key] = h
-        cap = 1 + 32 * 80
-        proof, V = C.create_string_buffer(cap), C.create_string_buffer(96)
-        c0 = ctxs[0]
-        rc = c0.lib.bpg_r1cs_prove(c0.h, handles[0][key], inst["label"], len(inst["label"]), inst["aL"], inst["aR"], inst["aO"], inst["vals"], inst["blinds"],
-                                   bytes(32), 0, V, proof, cap)
-        assert rc > 0
-        proofs[key] = (proof.raw[:rc], V.raw)
-    keys = [(100 + (k % 5) * 90, (k % 101 == 7), k % 40) for k in range(total)]
+    # circuits and proofs on context 0 (verification only needs the device: any context of it will do)
+    c0 = ctxs[0]
+    wit = [(n, m, wp, wv, wc, v, inL, inR) for (k, label, n, m, rp, tv, tc, (inL, inR, wp, wv, wc), v, vb, valid) in built]
+    handles = c0.circuit_create_batch([(n, m, rp, tv, tc) for (k, label, n, m, rp, tv, tc, _, v, vb, valid) in built])
+    items, expected = [], []
+    for b0 in range(0, len(built), 256):
+        chunk = range(b0, min(len(built), b0 + 256))
+        ws = c0.witness_eval_batch([wit[i] for i in chunk])
+        got = c0.prove_batch([(handles[i], built[i][1], w[0], w[1], w[2], built[i][8], built[i][9], hashlib.sha256(b"cfg5 ext %d" % built[i][0]).digest())
+                              for i, w in zip(chunk, ws)])
+        for i, (proof, V) in zip(chunk, got):
+            items.append((handles[i], built[i][1], V, proof, hashlib.sha256(b"cfg5 verify ext %d" % built[i][0]).digest()))
+            expected.append(built[i][10])
 
-    def lane(ci):
-        c = ctxs[ci]
-        out = []
-        for k in range(ci, total, K):
-            key = keys[k]
-            inst = shapes[key]
-            proof, V = proofs[key]
-            acc = C.c_int(-1)
-            c.check(c.lib.bpg_r1cs_verify(c.h, handles[ci][key], inst["label"], len(inst["label"]), V, proof, len(proof), bytes(32), 0, C.byref(acc)))
-            out.append((k, bool(acc.value)))
-        return out
+    def timed(idx_set, B):
+        calls = [idx_set[b:b + B] for b in range(0, len(idx_set), B)]
+        out = {}
 
-    def lane_batched(ci, B=64):
-        c = ctxs[ci]
-        out = []
-        mine = list(range(ci, total, K))
-        for b0 in range(0, len(mine), B):
-            ks = mine[b0:b0 + B]
-            batch = [(handles[ci][keys[k]], shapes[keys[k]]["label"], proofs[keys[k]][1], proofs[keys[k]][0], bytes([k % 251]) * 32) for k in ks]
-            out += list(zip(ks, c.verify_batch(batch)))
-        return out
+        def lane(ci):
+            c = ctxs[ci]
+            for chunk in calls[ci::NCTX]:
+                for i, acc in zip(chunk, c.verify_batch([items[i] for i in chunk])):
+                    out[i] = acc
+        for c in ctxs:
+            c.sync()
+        l0 = sum(c.launch_count() for c in ctxs)
+        cpu0, t0 = time.process_time(), time.perf_counter()
+        with ThreadPoolExecutor(NCTX) as tp:
+            list(tp.map(lane, range(NCTX)))
+        for c in ctxs:
+            c.sync()
+        dt, cpu = time.perf_counter() - t0, time.process_time() - cpu0
+        n = len(idx_set)
+        return out, {"verifications_per_sec": n / dt, "seconds": dt, "launches_per_verification": (sum(c.launch_count() for c in ctxs) - l0) / n,
+                     "host_cpu_ms_per_verification": 1e3 * cpu / n}
 
-    pool = ThreadPoolExecutor(max_workers=K)
-    list(pool.map(lane, range(K)))  # warm-up
-    t0 = time.perf_counter()
-    res = list(pool.map(lane, range(K)))
-    dt = time.perf_counter() - t0
-    verdicts = dict(x for r in res for x in r)
-    ok = all(verdicts[k] == items[k][1] for k in range(total))
-    list(pool.map(lane_batched, range(K)))
-    t0 = time.perf_counter()
-    resb = list(pool.map(lane_batched, range(K)))
-    dtb = time.perf_counter() - t0
-    vb = dict(x for r in resb for x in r)
-    okb = all(vb[k] == items[k][1] for k in range(total))
-    print(json.dumps({"contexts": K, "proofs": total, "verifications_per_sec": total / dt, "batched_verifications_per_sec": total / dtb,
-                      "batched_verdicts_match_expected": okb, "batch_size": 64, "invalid": sum(1 for it in items if not it[1]),
-                      "verdicts_match_expected": ok}))
+    every = list(range(len(items)))
+    valid_only = [i for i in every if expected[i]]
+    runs, verdicts = {}, {}
+    for B in [int(x) for x in args.per_call.split(",")]:
+        for tag, idx_set in (("invalid_1pct", every), ("invalid_0pct", valid_only)):
+            timed(idx_set, B)  # warm-up at this shape (the first call of a shape grows the scratch buffers)
+            reps = [timed(idx_set, B) for _ in range(args.repeat)]
+            got = reps[-1][0]
+            rates = sorted(r[1]["verifications_per_sec"] for r in reps)
+            runs["per_call_%d_%s" % (B, tag)] = {"verifications": len(idx_set), "invalid": sum(1 for i in idx_set if not expected[i]),
+                                                  "median_verifications_per_sec": rates[len(rates) // 2], "runs": [r[1] for r in reps],
+                                                  "verdicts_match_expected": all(got[i] == expected[i] for i in idx_set)}
+            verdicts.update(got)
+    digest = hashlib.sha256(bytes(int(verdicts[i]) for i in every)).hexdigest()
+    result = {"gpu": name, "power_limit": power, "statements": len(items),
+              "invalid_statements": expected.count(False), "contexts": NCTX, "runs": runs, "verdict_digest": digest}
+    for h in handles:
+        c0.lib.bpg_circuit_destroy(h)
+    for c in ctxs:
+        c.close()
+    line = json.dumps(result)
+    print(line)
+    if args.out:
+        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+        with open(args.out, "w") as f:
+            f.write(line + "\n")
 
 
 if __name__ == "__main__":
