@@ -62,6 +62,8 @@ SYMBOLS = {
     "bpg_r1cs_verify": (_i32, [_vp, _vp, _u8p, _sz, _u8p, _u8p, _sz, _u8p, C.c_uint, C.POINTER(_i32)]),
     "bpg_r1cs_verify_batch": (_i32, [_vp, _sz, C.POINTER(_vp), C.POINTER(C.c_char_p), C.POINTER(_sz), C.POINTER(C.c_char_p), C.POINTER(C.c_char_p),
                                      C.POINTER(_sz), _u8p, C.c_uint, C.POINTER(_i32)]),
+    "bpg_r1cs_verify_each": (_i32, [_vp, _sz, C.POINTER(_vp), C.POINTER(C.c_char_p), C.POINTER(_sz), C.POINTER(C.c_char_p), C.POINTER(C.c_char_p),
+                                    C.POINTER(_sz), _u8p, C.c_uint, C.POINTER(_i32)]),
     "bpg_transcript_new": (_vp, [_u8p, _sz]),
     "bpg_transcript_free": (None, [_vp]),
     "bpg_transcript_append": (None, [_vp, _u8p, _sz, _u8p, _sz]),

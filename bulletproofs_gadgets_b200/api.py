@@ -221,7 +221,16 @@ class Context:
     # ---- batch verification
     def verify_batch(self, items, flags=0):
         """items: list of (circuit handle (c_void_p), label bytes, V bytes, proof bytes, ext_rng32) -> list of bool,
-        verdict i being exactly what bpg_r1cs_verify returns for item i"""
+        verdict i being exactly what bpg_r1cs_verify returns for item i (one combined check with random weights; if it fails,
+        one check per proof)"""
+        return self._verify_many(self.lib.bpg_r1cs_verify_batch, items, flags)
+
+    def verify_each(self, items, flags=0):
+        """items as for verify_batch -> list of bool, verdict i being exactly what bpg_r1cs_verify returns for item i: every
+        proof is checked against its own verification equation (bpg_r1cs_verify_each), whatever the other proofs are"""
+        return self._verify_many(self.lib.bpg_r1cs_verify_each, items, flags)
+
+    def _verify_many(self, fn, items, flags):
         n = len(items)
         if n == 0:
             return []
@@ -233,7 +242,7 @@ class Context:
         plens = (C.c_size_t * n)(*[len(it[3]) for it in items])
         ext = b"".join(it[4] for it in items)
         acc = (C.c_int * n)()
-        self.check(self.lib.bpg_r1cs_verify_batch(self.h, n, circs, labels, lens, Vs, proofs, plens, ext, flags, acc))
+        self.check(fn(self.h, n, circs, labels, lens, Vs, proofs, plens, ext, flags, acc))
         return [bool(a) for a in acc]
 
     # ---- misc
@@ -617,19 +626,30 @@ def verify_batch(verifiers, proofs, ext_rngs=None, flags=0):
     """Verifier::verify of many statements in ONE call (bpg_r1cs_verify_batch) -> list of bool, entry i being whether
     verifiers[i].verify(proofs[i], ext_rng32=ext_rngs[i], flags=flags) succeeds.  The verifiers share one context; their
     circuits are made by one bpg_circuit_create_batch.  ext_rngs (one 32-byte string per verifier) default to os.urandom."""
+    return _verify_many("verify_batch", verifiers, proofs, ext_rngs, flags)
+
+
+def verify_each(verifiers, proofs, ext_rngs=None, flags=0):
+    """As verify_batch, through bpg_r1cs_verify_each: every proof is checked against its own verification equation, so entry i
+    is exactly verifiers[i].verify(proofs[i], ext_rng32=ext_rngs[i], flags=flags)'s outcome whatever the other proofs are,
+    at a cost that does not depend on how many of them are false."""
+    return _verify_many("verify_each", verifiers, proofs, ext_rngs, flags)
+
+
+def _verify_many(name, verifiers, proofs, ext_rngs, flags):
     if len(proofs) != len(verifiers):
-        raise ValueError("verify_batch: %d proofs for %d verifiers" % (len(proofs), len(verifiers)))
+        raise ValueError("%s: %d proofs for %d verifiers" % (name, len(proofs), len(verifiers)))
     if not verifiers:
         return []
     ctx = verifiers[0].ctx
     if any(v.ctx is not ctx for v in verifiers):
-        raise ValueError("verify_batch: every verifier must use the same Context")
+        raise ValueError("%s: every verifier must use the same Context" % name)
     exts = list(ext_rngs) if ext_rngs is not None else [os.urandom(32) for _ in verifiers]
     if len(exts) != len(verifiers):
-        raise ValueError("verify_batch: %d ext_rngs for %d verifiers" % (len(exts), len(verifiers)))
+        raise ValueError("%s: %d ext_rngs for %d verifiers" % (name, len(exts), len(verifiers)))
     circs = ctx.circuit_create_batch([v._circuit_args(len(v.V)) for v in verifiers])
     try:
-        return ctx.verify_batch([(c, v.label, b"".join(v.V), bytes(pf), ext) for c, v, pf, ext in zip(circs, verifiers, proofs, exts)], flags)
+        return getattr(ctx, name)([(c, v.label, b"".join(v.V), bytes(pf), ext) for c, v, pf, ext in zip(circs, verifiers, proofs, exts)], flags)
     finally:
         for c in circs:
             ctx.lib.bpg_circuit_destroy(c)

@@ -282,6 +282,65 @@ __global__ void __launch_bounds__(128) k_pb_axpy_gh(const vb_term *__restrict__ 
     st_sc(&acc[t], a);
 }
 
+// ---- per-proof check of a pass (verify_check_pass, verify_batch.inl): every proof against its own verification equation.
+// The own-point terms of the pass are concatenated, proof p owning terms [toff[p], toff[p+1]) (at least 11 each), t2p[t] =
+// proof of term t.  Variable-base part, one thread per term: decode (a failure clears ok[p] of that proof only), windowed
+// scalar multiplication, then one block sum per proof the block touches -> part[block + p].  Consecutive blocks share at most
+// one proof, so block + p is unique per (block, proof) pair and part holds blocks + K points.
+__global__ void __launch_bounds__(64) k_pb_varbase(const sc *__restrict__ es, const uint8_t *__restrict__ ep, const uint32_t *__restrict__ t2p, uint32_t k,
+                                                   uint32_t *__restrict__ ok, ge *__restrict__ part) {
+    __shared__ ge smem[64];
+    const uint32_t t0 = blockIdx.x * 64u, t = t0 + threadIdx.x;
+    const uint32_t q0 = t2p[t0], q1 = t2p[min(t0 + 63u, k - 1u)];
+    uint32_t q = 0xFFFFFFFFu;
+    ge acc;
+    ge_identity(acc);
+    if (t < k) {
+        q = t2p[t];
+        uint8_t b[32];
+        for (int i = 0; i < 32; i++) b[i] = ep[32ull * t + i];
+        ge p;
+        if (ristretto_decode(p, b)) {
+            sc s;
+            ld_sc(s, &es[t]);
+            sc_reduce(s, s);
+            ge_scalarmul_w4(acc, s, p);
+        } else atomicAnd(&ok[q], 0u);
+    }
+#pragma unroll 1
+    for (uint32_t r = q0; r <= q1; r++) {
+        ge x;
+        if (q == r) x = acc; else ge_identity(x);
+        block_sum_points(x, smem);
+        if (threadIdx.x == 0) st_ge(&part[blockIdx.x + r], x);
+    }
+}
+// one block per proof: its variable-base partials + its fixed-base output, verdict[p] = decoded && identity (all-zero encoding),
+// the test verify_finish applies to one proof
+__global__ void __launch_bounds__(64) k_pb_check_out(const uint32_t *__restrict__ toff, const ge *__restrict__ fixed, const ge *__restrict__ part,
+                                                     const uint32_t *__restrict__ ok, int *__restrict__ verdict) {
+    __shared__ ge smem[64];
+    const uint32_t p = blockIdx.x, b0 = toff[p] / 64u, b1 = (toff[p + 1] - 1u) / 64u;
+    ge acc;
+    ge_identity(acc);
+#pragma unroll 1
+    for (uint32_t b = b0 + threadIdx.x; b <= b1; b += 64u) {
+        ge x;
+        ld_ge(x, &part[b + p]);
+        ge_add(acc, acc, x);
+    }
+    block_sum_points(acc, smem);
+    if (threadIdx.x == 0) {
+        ge f;
+        ld_ge(f, &fixed[p]);
+        ge_add(acc, acc, f);
+        uint8_t e[32], nz = 0;
+        ristretto_encode(e, acc);
+        for (int i = 0; i < 32; i++) nz |= e[i];
+        verdict[p] = (ok[p] && nz == 0) ? 1 : 0;
+    }
+}
+
 // ---- many-output small MSM (msm_run_many): k_msm_digits<*, SPLIT = 1> with the segments in a device table (any number of
 // them, ascending `start`) and one bucket group per output, so the group count is not bounded by msm_params
 template <int SCATTER>

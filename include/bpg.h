@@ -224,17 +224,31 @@ int bpg_r1cs_verify(bpg_ctx *ctx, bpg_circuit *c, const uint8_t *label, size_t l
 
 /* Batch verification (SURVEY 8 f-4): accept[i] = what bpg_r1cs_verify returns for proof i.  The proofs are combined
  * with random weights into ONE fixed-base multiscalar multiplication over the resident generators plus one
- * variable-base launch over all proofs' own points; a failing combination is bisected until the invalid proofs are
- * isolated, so verdicts equal one-by-one verification.  ext_rng32 = count x 32 bytes (one thread_rng stand-in per proof):
+ * variable-base launch over all proofs' own points.  If that combined check fails, every proof of the call is checked on
+ * its own as by bpg_r1cs_verify_each (no bisection), so whenever any proof of the call is false the verdicts are exactly
+ * one-by-one verification's; an all-valid call is accepted up to the 2^-250 soundness error of the weights, which depend
+ * on every proof of the call.  bpg_r1cs_verify_each is the exact choice at any rate of false proofs; this entry is the
+ * cheaper one when false proofs are rare.  ext_rng32 = count x 32 bytes (one thread_rng stand-in per proof):
  * it MUST be fresh secret randomness (the reference draws it from thread_rng inside Verifier::verify).  The combination
  * weights are derived from every proof's label, commitments and full proof bytes together with ext_rng32, so they are
  * bound to the statements being checked and cannot be anticipated by the provers.  Every transcript is replayed on the
  * host; the proofs whose replay succeeds and whose padded size N is at most 4096 have their scalars prepared in lockstep,
  * in passes of at most 1 024 proofs and 2^17 padded elements with a fixed number of launches each, larger proofs one by
- * one inside the call.  Each combined check of a set of proofs sums their G/H scalars in one launch. */
+ * one inside the call.  The combined check sums the G/H scalars of all proofs in one launch.  count = 0 returns BPG_OK; a
+ * NULL array, or a NULL entry where bpg_r1cs_verify needs a pointer, returns BPG_E_ARG with accept zeroed. */
 int bpg_r1cs_verify_batch(bpg_ctx *ctx, size_t count, bpg_circuit *const *circuits, const uint8_t *const *labels,
                           const size_t *label_lens, const uint8_t *const *V32, const uint8_t *const *proofs,
                           const size_t *proof_lens, const uint8_t *ext_rng32, unsigned flags, int *accept);
+/* K independent verifications in one call: accept[i] = what
+ *   bpg_r1cs_verify(ctx, circuits[i], labels[i], label_lens[i], V32[i], proofs[i], proof_lens[i], ext_rng32 + 32 i, flags, ...)
+ * returns, exactly: every proof is checked against its OWN verification equation (no weights across proofs), so a verdict depends
+ * on that proof and its ext_rng32 alone.  Replayed proofs of padded N <= 4096 are prepared and checked in lockstep passes (at most
+ * 1 024 proofs, 2^17 padded elements and 2^17 own points each) with a fixed set of launches per pass and one read-back per call;
+ * larger proofs are verified as bpg_r1cs_verify does inside the call.  The launches depend on the proofs' sizes, not on which of
+ * them are false.  Arguments, flags, count = 0 and errors as for bpg_r1cs_verify_batch. */
+int bpg_r1cs_verify_each(bpg_ctx *ctx, size_t count, bpg_circuit *const *circuits, const uint8_t *const *labels,
+                         const size_t *label_lens, const uint8_t *const *V32, const uint8_t *const *proofs,
+                         const size_t *proof_lens, const uint8_t *ext_rng32, unsigned flags, int *accept);
 
 /* Merlin transcript (host; sequential Keccak, never on the device) exposed for the Rust shim and the tests */
 typedef struct bpg_transcript bpg_transcript;

@@ -66,6 +66,7 @@ extern "C" {
     pub fn bpg_r1cs_prove_batch(ctx: *mut BpgCtx, count: usize, circuits: *const *mut BpgCircuit, labels: *const *const u8, label_lens: *const usize, aL: *const *const u8, aR: *const *const u8, aO: *const *const u8, v: *const *const u8, v_blinding: *const *const u8, ext_rng32: *const u8, flags: u32, V_out: *const *mut u8, proofs: *const *mut u8, proof_caps: *const usize, proof_lens: *mut usize) -> i32;
     pub fn bpg_r1cs_verify(ctx: *mut BpgCtx, c: *mut BpgCircuit, label: *const u8, label_len: usize, V32: *const u8, proof: *const u8, proof_len: usize, ext_rng32: *const u8, flags: u32, accept: *mut i32) -> i32;
     pub fn bpg_r1cs_verify_batch(ctx: *mut BpgCtx, count: usize, circuits: *const *mut BpgCircuit, labels: *const *const u8, label_lens: *const usize, V32: *const *const u8, proofs: *const *const u8, proof_lens: *const usize, ext_rng32: *const u8, flags: u32, accept: *mut i32) -> i32;
+    pub fn bpg_r1cs_verify_each(ctx: *mut BpgCtx, count: usize, circuits: *const *mut BpgCircuit, labels: *const *const u8, label_lens: *const usize, V32: *const *const u8, proofs: *const *const u8, proof_lens: *const usize, ext_rng32: *const u8, flags: u32, accept: *mut i32) -> i32;
     pub fn bpg_transcript_new(label: *const u8, len: usize) -> *mut BpgTranscript;
     pub fn bpg_transcript_free(t: *mut BpgTranscript);
     pub fn bpg_transcript_append(t: *mut BpgTranscript, label: *const u8, ll: usize, msg: *const u8, ml: usize);

@@ -53,6 +53,15 @@ pub struct ProveJob<'a> {
     pub v_blinding: &'a [u8],
 }
 
+/// One statement of Device::r1cs_verify_each: the arguments of one Device::r1cs_verify call.
+pub struct VerifyJob<'a> {
+    pub label: &'a [u8],
+    pub cs: &'a FlatConstraints,
+    pub n: usize,
+    pub commitments: &'a [u8],
+    pub proof: &'a [u8],
+}
+
 pub const VAR_L: u32 = 0;
 pub const VAR_R: u32 = 1;
 pub const VAR_O: u32 = 2;
@@ -217,6 +226,38 @@ impl Device {
         };
         unsafe { ffi::bpg_circuit_destroy(circuit) };
         self.check(rc).map(|_| accept == 1)
+    }
+    /// Verifier::verify for many statements in one call (bpg_r1cs_verify_each): entry i is exactly what r1cs_verify returns for
+    /// jobs[i]; every proof is checked against its own equation, small ones (padded size <= 4096) in lockstep.
+    pub fn r1cs_verify_each(&mut self, jobs: &[VerifyJob], flags: u32) -> Result<Vec<bool>, BpgError> {
+        use rand::RngCore;
+        let k = jobs.len();
+        let mut ext = vec![0u8; 32 * k];
+        rand::thread_rng().fill_bytes(&mut ext);
+        let ns: Vec<usize> = jobs.iter().map(|j| j.n).collect();
+        let ms: Vec<usize> = jobs.iter().map(|j| j.commitments.len() / 32).collect();
+        let qs: Vec<usize> = jobs.iter().map(|j| j.cs.rows()).collect();
+        let row_ptrs: Vec<*const u32> = jobs.iter().map(|j| j.cs.row_ptr.as_ptr()).collect();
+        let term_vars: Vec<*const u32> = jobs.iter().map(|j| j.cs.term_var.as_ptr()).collect();
+        let term_coeffs: Vec<*const u8> = jobs.iter().map(|j| j.cs.term_coeff.as_ptr()).collect();
+        let mut circuits: Vec<*mut ffi::BpgCircuit> = vec![ptr::null_mut(); k];
+        let rc = unsafe {
+            ffi::bpg_circuit_create_batch(self.ctx, k, ns.as_ptr(), ms.as_ptr(), qs.as_ptr(), row_ptrs.as_ptr(), term_vars.as_ptr(), term_coeffs.as_ptr(),
+                                          circuits.as_mut_ptr())
+        };
+        self.check(rc)?;
+        let labels: Vec<*const u8> = jobs.iter().map(|j| j.label.as_ptr()).collect();
+        let label_lens: Vec<usize> = jobs.iter().map(|j| j.label.len()).collect();
+        let vs: Vec<*const u8> = jobs.iter().map(|j| j.commitments.as_ptr()).collect();
+        let proofs: Vec<*const u8> = jobs.iter().map(|j| j.proof.as_ptr()).collect();
+        let proof_lens: Vec<usize> = jobs.iter().map(|j| j.proof.len()).collect();
+        let mut accept = vec![0i32; k];
+        let rc = unsafe {
+            ffi::bpg_r1cs_verify_each(self.ctx, k, circuits.as_ptr(), labels.as_ptr(), label_lens.as_ptr(), vs.as_ptr(), proofs.as_ptr(),
+                                      proof_lens.as_ptr(), ext.as_ptr(), flags, accept.as_mut_ptr())
+        };
+        for c in &circuits { unsafe { ffi::bpg_circuit_destroy(*c) } }
+        self.check(rc).map(|_| accept.iter().map(|&a| a == 1).collect())
     }
     /// install ROUND_CONSTANTS_769 (mimc_consts.rs:2-489) once: 486 x 32 bytes
     pub fn mimc_set_constants(&mut self, consts: &[u8]) -> Result<(), BpgError> {
