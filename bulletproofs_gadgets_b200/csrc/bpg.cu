@@ -662,7 +662,7 @@ int msm_materialise_fold(bpg_ctx *ctx, cudaStream_t s, uint32_t N, uint32_t npri
         else if (scatter) k_mat_digits<1><<<LAUNCH_1D(nt, 256), 0, s>>>(N, nprime, cap, ptotal, d_EG, d_EH, p0, p1, cc, sorted);
         else k_mat_digits<0><<<LAUNCH_1D(nt, 256), 0, s>>>(N, nprime, cap, ptotal, d_EG, d_EH, p0, p1, cc, sorted);
     }));
-    k_mat_reduce<<<nout, 32, 0, s>>>((const ge *)ctx->buckets.p, nout, (ge *)ctx->mat_pts.p);
+    k_mat_reduce<<<LAUNCH_1D(2 * nout, 64), 0, s>>>((const ge *)ctx->buckets.p, nout, (ge *)ctx->mat_pts.p);
     KCHECK();
     if (sharded) CTX_TRY(shard_exchange_sum(ctx, s, (ge *)ctx->mat_pts.p, nout));
     k_mat_chain<<<LAUNCH_1D(nout, 64), 0, s>>>((const ge *)ctx->mat_pts.p, nout, (ge *)ctx->mat_ext.p);

@@ -41,7 +41,7 @@ typedef struct bpg_circuit bpg_circuit;
 #define BPG_FLAG_WITNESS_ON_DEVICE 4u /* aL, aR, aO are device pointers to reduced scalars (HBM-resident timing) */
 #define BPG_FLAG_FAST_BLINDING 2u  /* s_L, s_R expanded on the device from a transcript-derived seed instead of
                                       2n sequential Merlin TranscriptRng draws: valid proofs, different bytes */
-/* Inner-product argument: after the first rounds the folded generators G^(k), H^(k) (512 each) are materialised once by a
+/* Inner-product argument: after the first rounds the folded generators G^(k), H^(k) (512 each, N/64 for large unsharded proofs) are materialised once by a
  * multi-output MSM and the remaining rounds run over them (same L_j, R_j bytes, ~1/3 fewer point additions per proof).
  * On by default for padded sizes >= 2^15; these two flags force it off / on (any size >= 4) for tests and A/B timing. */
 #define BPG_FLAG_NO_LATE_FOLD 8u
